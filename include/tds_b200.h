@@ -233,13 +233,20 @@ typedef struct {
     int32_t reserved;
 } tds_map_info_t;
 int tds_map_info(const tds_map_t* map, tds_map_info_t* out);
+/* The offroad distance bound of a map (what tds_offroad_fwd uses to settle on-road corners without a search):
+ * h_geom[4] = x0, y0 of the grid, subcell size, metres per code unit; h_dims[2] = gx, gy; h_codes [gy][gx] u8 or NULL.
+ * Code q < 255: every point of the subcell lies within q * h_geom[3] metres of the mesh by the reference's fp32
+ * distance; 255: unknown.  Synchronous copy. */
+int tds_map_offroad_bound(const tds_map_t* map, float* h_geom, int32_t* h_dims, uint8_t* h_codes);
 
 /* ------------------------------------------------------------------------------------------
  * Offroad.  Replaces offroad_infraction_loss (infractions.py:176-229) + point_to_mesh_distance_pt
  * (infractions.py:86-173): out[b,a] = sum over the 4 box corners of (d2 if d2 > threshold else 0),
  * d2 = min over ALL map faces of the reference's squared point-triangle distance; times present.
  * maps[d_env_map[b]] is the map of environment b (d_env_map NULL: map 0 for all).
- * d_face [B,A,4] int32 or NULL receives the argmin face per corner (for the backward).
+ * d_face [B,A,4] int32 or NULL receives the argmin face per corner (for the backward); -1 for a corner with no
+ * gradient that needed no search: absent, or settled by the map's distance bound (d2 <= threshold).  The environment
+ * variable TDS_OFFROAD_TRIAGE=0 searches every corner (same d_out).
  * ---------------------------------------------------------------------------------------- */
 int tds_offroad_fwd(const tds_map_t* const* maps, int32_t n_maps, const int32_t* d_env_map,
                     const float* d_state, const float* d_lenwid, const uint8_t* d_present,

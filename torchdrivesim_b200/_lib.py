@@ -83,6 +83,7 @@ SIGNATURES = {
     "tds_map_create": (c_void_p, [c_void_p, c_int32, c_void_p, c_int32, c_void_p, c_float, c_float]),
     "tds_map_destroy": (None, [c_void_p]),
     "tds_map_info": (c_int32, [c_void_p, POINTER(MapInfo)]),
+    "tds_map_offroad_bound": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "tds_offroad_fwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                   c_float, c_void_p, c_void_p, c_void_p]),
     "tds_offroad_bwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,

@@ -12,6 +12,7 @@
 //         out[b,i] = sum_j o_ij m_j - max_j o_ij m_j, one warp per row i, lanes over columns j,
 //         warp-shuffle reductions; per-environment box data staged in shared memory.
 // This work is FP32-pipe bound (no HBM traffic to speak of: 20 B per box in, 4 B per row out).
+#include <cooperative_groups.h>
 #include <math_constants.h>
 
 #include "tds_common.cuh"
@@ -277,13 +278,23 @@ __global__ void __launch_bounds__(128) sensing_occlusion_kernel(const float4* __
 
 // ---- aggregate infraction metrics of a step (the vector that is all-reduced over the GPUs, SURVEY.md §8e):
 // acc[0..5] += sum of collision over present agents, sum of offroad, agents with collision > 0, agents with
-// offroad > 0, present agents, agent slots.  ONE CTA with a fixed reduction order: the sums are reproducible.
-__global__ void __launch_bounds__(1024) infraction_metrics_kernel(const float* __restrict__ collision, const float* __restrict__ offroad,
-                                                                  const uint8_t* __restrict__ present, int64_t n,
-                                                                  double* __restrict__ acc) {
+// offroad > 0, present agents, agent slots.  One cluster of kMetricCtas CTAs with a fixed reduction order: thread t of
+// the cluster sums elements t, t + 8192, ... in order, then warps (shuffle tree), the 32 warps of a CTA and the CTAs of
+// the cluster (in CTA 0's shared memory) are summed in index order.  The sums are reproducible run to run; the counts
+// are exact.  Versions that reduced in one CTA summed in another order: their float64 sums differ from these in the last
+// bits, the counts are the same.
+constexpr int kMetricCtas = 8;
+__global__ void __cluster_dims__(kMetricCtas, 1, 1) __launch_bounds__(1024)
+infraction_metrics_kernel(const float* __restrict__ collision, const float* __restrict__ offroad,
+                          const uint8_t* __restrict__ present, int64_t n, double* __restrict__ acc) {
+    namespace cg = cooperative_groups;
+    cg::cluster_group cluster = cg::this_cluster();
     __shared__ double s_part[32][5];
+    __shared__ double s_cta[kMetricCtas][5];          // used in CTA 0: one row per CTA of the cluster
+    const int rank = (int)cluster.block_rank();
     double v[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
-    for (int64_t i = threadIdx.x; i < n; i += blockDim.x) {
+    const int64_t stride = (int64_t)kMetricCtas * blockDim.x;
+    for (int64_t i = (int64_t)rank * blockDim.x + threadIdx.x; i < n; i += stride) {
         const bool here = present ? present[i] != 0 : true;
         const float c = collision[i], o = offroad[i];
         if (here) { v[0] += (double)c; v[1] += (double)o; v[2] += c > 0.0f; v[3] += o > 0.0f; v[4] += 1.0; }
@@ -299,9 +310,15 @@ __global__ void __launch_bounds__(1024) infraction_metrics_kernel(const float* _
     if (threadIdx.x < 5) {
         double t = 0.0;
         for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += s_part[w][threadIdx.x];
+        cluster.map_shared_rank(&s_cta[0][0], 0)[rank * 5 + threadIdx.x] = t;
+    }
+    cluster.sync();
+    if (rank == 0 && threadIdx.x < 5) {
+        double t = 0.0;
+        for (int r = 0; r < kMetricCtas; r++) t += s_cta[r][threadIdx.x];
         acc[threadIdx.x] += t;
     }
-    if (threadIdx.x == 5) acc[5] += (double)n;
+    if (rank == 0 && threadIdx.x == 5) acc[5] += (double)n;
 }
 
 // ---- IoU backward.  d(intersection area) is the boundary integral of the normal velocity: every edge of
@@ -665,7 +682,7 @@ extern "C" int tds_infraction_metrics(const float* d_collision, const float* d_o
                                       int64_t n, double* d_acc, void* stream) {
     TDS_REQUIRE(n >= 0, "infraction_metrics: negative size");
     TDS_REQUIRE(d_acc && (n == 0 || (d_collision && d_offroad)), "infraction_metrics: null pointer");
-    infraction_metrics_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(d_collision, d_offroad, d_present, n, d_acc);
+    infraction_metrics_kernel<<<kMetricCtas, 1024, 0, (cudaStream_t)stream>>>(d_collision, d_offroad, d_present, n, d_acc);
     TDS_LAUNCH_OK();
     return TDS_OK;
 }

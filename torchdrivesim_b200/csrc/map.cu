@@ -355,6 +355,27 @@ extern "C" tds_map_t* tds_map_create(const float* h_verts, int32_t nv, const int
     d.scell = (const int32_t*)m->allocations[7];
     d.rec_all = (const float4*)m->allocations[8];
     d.rcell_all = (const int32_t*)m->allocations[9];
+    // ---------------- offroad distance bound (computed on the device from the offroad grid just uploaded)
+    d.bcs = 0.25f;
+    d.bx0 = minx - 1.0f;
+    d.by0 = miny - 1.0f;
+    auto nsub = [&](float lo, float hi) { return (int64_t)std::floor(((double)hi + 1.0 - lo) / d.bcs) + 1; };
+    while (nsub(d.bx0, maxx) * nsub(d.by0, maxy) > ((int64_t)16 << 20)) d.bcs *= 2.0f;
+    d.binv = 1.0f / d.bcs;
+    d.bgx = (int32_t)nsub(d.bx0, maxx);
+    d.bgy = (int32_t)nsub(d.by0, maxy);
+    const size_t nb = (size_t)d.bgx * d.bgy;
+    if (cudaMalloc(&m->allocations[10], nb) != cudaSuccess) {
+        fail(TDS_ERR_CUDA, "map_create: device allocation failed: %s", cudaGetErrorString(cudaGetLastError()));
+        tds_map_destroy(m);
+        return nullptr;
+    }
+    if (offroad_bound_build(d, (uint8_t*)m->allocations[10]) != TDS_OK) {     // the error is recorded by the builder
+        tds_map_destroy(m);
+        return nullptr;
+    }
+    bytes += (int64_t)nb;
+    d.obound = (const uint8_t*)m->allocations[10];
     m->info.n_verts = nv; m->info.n_faces = nf;
     m->info.raster_gx = d.rgx; m->info.raster_gy = d.rgy; m->info.raster_records = n_recs; m->info.raster_strips = (int32_t)srecs.size();
     m->info.offroad_gx = d.ogx; m->info.offroad_gy = d.ogy;
@@ -373,5 +394,15 @@ extern "C" void tds_map_destroy(tds_map_t* map) {
 extern "C" int tds_map_info(const tds_map_t* map, tds_map_info_t* out) {
     TDS_REQUIRE(map && out, "map_info: null pointer");
     *out = map->info;
+    return TDS_OK;
+}
+
+extern "C" int tds_map_offroad_bound(const tds_map_t* map, float* h_geom, int32_t* h_dims, uint8_t* h_codes) {
+    TDS_REQUIRE(map && h_geom && h_dims, "map_offroad_bound: null pointer");
+    const tds::MapDev& d = map->dev;
+    h_geom[0] = d.bx0; h_geom[1] = d.by0; h_geom[2] = d.bcs; h_geom[3] = 1.0f / tds::kBoundPerMetre;
+    h_dims[0] = d.bgx; h_dims[1] = d.bgy;
+    if (h_codes && cudaMemcpy(h_codes, d.obound, (size_t)d.bgx * d.bgy, cudaMemcpyDeviceToHost) != cudaSuccess)
+        return tds::fail(TDS_ERR_CUDA, "map_offroad_bound: copy failed: %s", cudaGetErrorString(cudaGetLastError()));
     return TDS_OK;
 }

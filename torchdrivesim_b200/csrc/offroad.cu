@@ -2,12 +2,14 @@
 //
 // Reference: offroad_infraction_loss (torchdrivesim/infractions.py:176-229, pure-torch branch) and
 // point_to_mesh_distance_pt (infractions.py:86-173), which expand the mesh to a
-// [B*A*4, F, 3, 3] tensor (290 TB at 1024 x 64 agents on Town01).  Here one thread owns one
-// corner and walks the per-map uniform grid in expanding rings; the per-face arithmetic is the
+// [B*A*4, F, 3, 3] tensor (290 TB at 1024 x 64 agents on Town01).  Here a corner that the per-map
+// distance bound places within the threshold is settled at once; the others are searched by a warp that
+// walks the per-map uniform grid in expanding rings; the per-face arithmetic is the
 // reference's, operation for operation (fp32, no FMA), so the minimum over the visited faces is
 // the reference's minimum over all faces.  The grid (~1 MB per map) is L2 resident; HBM traffic is
 // the 28 B per agent of state/size in and 4 B out.
 #include <algorithm>
+#include <cstdlib>
 #include <math_constants.h>
 
 #include "tds_map.cuh"
@@ -198,43 +200,137 @@ __device__ __forceinline__ void corner_of(const float* st, const float* lw, int 
     py = (ux * s + uy * c) + st[1];
 }
 
-// one CTA of 4 warps per agent, one warp per box corner
+// ---- distance bound of the map (MapDev::obound), built once by tds_map_create.
+//
+// The forward settles a corner without a search when the bound of its subcell says d2 <= thr: the loss of that corner
+// is then 0 (F.threshold) whatever its exact distance.  For that, the bound must hold for the distance the search would
+// compute, i.e. the reference's fp32 formula d_ref(p) = min over faces of g_f(p), g_f = 0 if the fp32 barycentric test
+// says "inside", else the fp32 edge distance.  d_ref itself cannot serve at the subcell centre c: for an ill-conditioned
+// face the fp32 barycentric test can say "inside" for a point metres away, so d_ref(c) = 0 would say nothing about
+// the other points of the subcell.  The centre is measured instead in double precision with a distance D' that counts
+// a face as a solid triangle only where the reference's inside test is reliable (below), and as its three edges
+// elsewhere.  D' is a minimum of distances to closed sets, so it is 1-Lipschitz, and for p in the subcell
+//   d_ref(p) <= D'(p) + kFp32Err + kInsideBand <= D'(c) + |p - c| + kFp32Err + kInsideBand,
+// |p - c| <= half diagonal + kLookupErr.  The stored code is that sum rounded up to 1/64 m:
+//   kLookupErr  1e-4 m: the corner is placed in its subcell from (px - x0) rounded to fp32, 3e-5 m at 400 m.
+//   kFp32Err    2e-3 m: the reference's fp32 edge distance (projection, clamp, closest point, squared norm) is off the
+//               exact one by a few eps times (|coordinates| + edge length), 3e-4 m for 400 m coordinates and 100 m edges.
+//   kInsideBand 1e-2 m: a face is solid for D' only if its area is >= 5.05e-3 (the reference skips faces under 5e-3) and
+//               the fp32 barycentric weights are accurate to dw with dw * L <= kInsideBand (L = longest edge): a point
+//               inside such a face is either found inside by the reference (g = 0) or lies within dw * L of an edge.
+//               The weights are ratios of products of four edge-length factors over (2 area)^2, so
+//               dw <= 40 eps L^4 / (2 area)^2 + 1e-8 / (2 area)^2 (the second term is the reference's +1e-8).
+// The slack, kSlack = 0.02 m, is larger than their sum; the margin it costs is small next to sqrt(thr) - half diagonal.
+// Only faces binned into the offroad cells within kReach of the centre are visited: a minimum over fewer faces is
+// still an upper bound, and any face nearer than the largest code that can be stored is among them.
+constexpr double kSlack = 0.02, kInsideBand = 1e-2, kReach = 4.0;
+
+__device__ double seg_dist2_d(double px, double py, double ax, double ay, double bx, double by) {
+    const double abx = bx - ax, aby = by - ay, l2 = abx * abx + aby * aby;
+    double t = l2 > 0.0 ? (abx * (px - ax) + aby * (py - ay)) / l2 : 0.0;
+    t = fmin(fmax(t, 0.0), 1.0);
+    const double dx = px - (ax + t * abx), dy = py - (ay + t * aby);
+    return dx * dx + dy * dy;
+}
+
+__device__ double bound_face_dist2(double px, double py, float4 a, float4 b) {
+    const double x0 = a.x, y0 = a.y, x1 = a.z, y1 = a.w, x2 = b.x, y2 = b.y;
+    const double e = fmin(fmin(seg_dist2_d(px, py, x0, y0, x1, y1), seg_dist2_d(px, py, x0, y0, x2, y2)),
+                          seg_dist2_d(px, py, x1, y1, x2, y2));
+    const double cz = (x1 - x0) * (y2 - y0) - (y1 - y0) * (x2 - x0);      // 2 * signed area
+    const double l2 = fmax(fmax((x1 - x0) * (x1 - x0) + (y1 - y0) * (y1 - y0), (x2 - x0) * (x2 - x0) + (y2 - y0) * (y2 - y0)),
+                           (x2 - x1) * (x2 - x1) + (y2 - y1) * (y2 - y1));
+    const double L = sqrt(l2), a4 = cz * cz;
+    const double dw = (40.0 * 5.960464477539063e-08 * l2 * l2 + 1e-8) / a4;
+    if (fabs(cz) >= 2.0 * 5.05e-3 && dw * L <= kInsideBand) {
+        const double o0 = (x1 - px) * (y2 - py) - (y1 - py) * (x2 - px);
+        const double o1 = (x2 - px) * (y0 - py) - (y2 - py) * (x0 - px);
+        const double o2 = (x0 - px) * (y1 - py) - (y0 - py) * (x1 - px);
+        const bool inside = cz > 0.0 ? (o0 >= 0.0 && o1 >= 0.0 && o2 >= 0.0) : (o0 <= 0.0 && o1 <= 0.0 && o2 <= 0.0);
+        if (inside) return 0.0;
+    }
+    return e;                                     // NaN for a face with a non-finite vertex: ignored by the caller
+}
+
+// one thread per subcell
+__global__ void __launch_bounds__(256) offroad_bound_kernel(MapDev m, uint8_t* __restrict__ obound) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)m.bgx * m.bgy) return;
+    const int sx = (int)(i % m.bgx), sy = (int)(i / m.bgx);
+    const double cx = (double)m.bx0 + ((double)sx + 0.5) * m.bcs, cy = (double)m.by0 + ((double)sy + 0.5) * m.bcs;
+    const int ix0 = max((int)floor((cx - kReach - m.ox0) / m.ocs), 0), ix1 = min((int)floor((cx + kReach - m.ox0) / m.ocs), m.ogx - 1);
+    const int iy0 = max((int)floor((cy - kReach - m.oy0) / m.ocs), 0), iy1 = min((int)floor((cy + kReach - m.oy0) / m.ocs), m.ogy - 1);
+    double best = CUDART_INF;
+    for (int y = iy0; y <= iy1; y++)
+        for (int x = ix0; x <= ix1; x++) {
+            const int c = y * m.ogx + x;
+            for (int e = m.ocell[c]; e < m.ocell[c + 1]; e++) {
+                const double d = bound_face_dist2(cx, cy, m.orec[2 * (int64_t)e], m.orec[2 * (int64_t)e + 1]);
+                if (d < best) best = d;
+            }
+        }
+    const double ub = sqrt(best) + 0.7071067811865476 * m.bcs + kSlack;          // +inf when no face was near
+    const double q = ceil(ub * tds::kBoundPerMetre);
+    obound[i] = q < (double)tds::kBoundUnknown ? (uint8_t)q : (uint8_t)tds::kBoundUnknown;
+}
+
+// the corner's squared distance is known to be <= thr from its subcell's bound (false for NaN, outside the grid, thr <= 0)
+__device__ __forceinline__ bool settled_by_bound(const MapDev& m, float px, float py, float thr) {
+    const float fx = (px - m.bx0) * m.binv, fy = (py - m.by0) * m.binv;
+    if (!(fx >= 0.0f && fy >= 0.0f && fx < (float)m.bgx && fy < (float)m.bgy)) return false;
+    const int q = __ldg(m.obound + (int64_t)(int)fy * m.bgx + (int)fx);
+    return q < tds::kBoundUnknown && (float)(q * q) <= thr * (float)(tds::kBoundPerMetre * tds::kBoundPerMetre);
+}
+
+// A warp holds 8 agents, lane l = corner l & 3 of agent 8 * group + l / 4.  Each lane places its corner and looks up the
+// map's distance bound: a corner whose bound is within the threshold is settled (value 0, face -1, the search would
+// have stopped at a face with d2 <= thr and returned 0 too).  The warp then searches the undecided corners one after
+// another with nearest_face, all 32 lanes on one corner.  Face -1 for a settled corner is what the backward needs: it
+// skips f < 0, and with the face of the search it would have skipped the corner as well (d2 <= thr); FusedRollout goes
+// through the same backward, and nothing else reads the face.  triage = false (TDS_OFFROAD_TRIAGE=0) searches every
+// corner: the values are the same, the faces of on-road corners are those of the search.
 #ifndef TDS_OFFROAD_MINB
-#define TDS_OFFROAD_MINB 12
+#define TDS_OFFROAD_MINB 4
 #endif
-__global__ void __launch_bounds__(128, TDS_OFFROAD_MINB) offroad_fwd_kernel(MapSetDev maps, const int32_t* __restrict__ env_map,
+__global__ void __launch_bounds__(256, TDS_OFFROAD_MINB) offroad_fwd_kernel(MapSetDev maps, const int32_t* __restrict__ env_map,
                                                           const float* __restrict__ state, const float* __restrict__ lenwid,
-                                                          const uint8_t* __restrict__ present, int B, int A, float thr,
+                                                          const uint8_t* __restrict__ present, int B, int A, float thr, bool triage,
                                                           float* __restrict__ out, int32_t* __restrict__ face) {
-    __shared__ float s_v[4];
-    __shared__ float2 s_corner[4];
-    const int lane = threadIdx.x & 31, k = threadIdx.x >> 5;
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31, k = lane & 3;
     const unsigned n_agents = (unsigned)B * (unsigned)A;          // < 2^31, checked by the host
-    for (unsigned agent = blockIdx.x; agent < n_agents; agent += gridDim.x) {
-    float v = 0.0f;
-    int bf = -1;
-    const int b = (int)(agent / (unsigned)A);
-    const bool here = present ? present[agent] != 0 : true;
-    if (here && threadIdx.x < 4) {                 // the (double precision) sin / cos is evaluated by 4 lanes of ONE warp
-        float px, py, s, c;
-        corner_of(state + 4 * (size_t)agent, lenwid + 2 * (size_t)agent, threadIdx.x, px, py, s, c);
-        s_corner[threadIdx.x] = make_float2(px, py);
-    }
-    __syncthreads();
-    if (here) {
-        const MapDev& m = maps.m[env_map ? env_map[b] : 0];
-        const float px = s_corner[k].x, py = s_corner[k].y;
-        const float d2 = nearest_face(m, px, py, fmaxf(thr, 0.0f), &bf, lane);
-        v = d2 > thr ? d2 : 0.0f;           // F.threshold(d2, thr, 0), infractions.py:172
-    }
-    if (lane == 0) {
-        if (face) face[4 * (size_t)agent + k] = bf;
-        s_v[k] = v;
-    }
-    __syncthreads();
-    // sum of the 4 corners, in corner order
-    if (threadIdx.x == 0) out[agent] = ((s_v[0] + s_v[1]) + s_v[2]) + s_v[3];
-    __syncthreads();
+    const unsigned n_groups = (n_agents + 7) / 8;
+    const unsigned n_warps = gridDim.x * (blockDim.x >> 5);
+    for (unsigned g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); g < n_groups; g += n_warps) {
+        const unsigned agent = 8 * g + (lane >> 2);
+        const bool valid = agent < n_agents;
+        const bool here = valid && (present ? present[agent] != 0 : true);
+        float v = 0.0f, px = 0.0f, py = 0.0f;
+        int bf = -1, mi = 0;
+        bool search = false;
+        if (here) {
+            float s, c;
+            corner_of(state + 4 * (size_t)agent, lenwid + 2 * (size_t)agent, k, px, py, s, c);
+            mi = env_map ? env_map[agent / (unsigned)A] : 0;
+            search = !(triage && settled_by_bound(maps.m[mi], px, py, thr));
+        }
+        for (unsigned todo = __ballot_sync(full, search); todo; todo &= todo - 1) {
+            const int src = __ffs(todo) - 1;
+            const int smi = __shfl_sync(full, mi, src);
+            const float sx = __shfl_sync(full, px, src), sy = __shfl_sync(full, py, src);
+            int sf;
+            const float d2 = nearest_face(maps.m[smi], sx, sy, fmaxf(thr, 0.0f), &sf, lane);
+            if (lane == src) {
+                v = d2 > thr ? d2 : 0.0f;           // F.threshold(d2, thr, 0), infractions.py:172
+                bf = sf;
+            }
+        }
+        if (valid && face) face[4 * (size_t)agent + k] = bf;
+        // sum of the 4 corners, in corner order
+        const int c0 = lane & ~3;
+        const float v0 = __shfl_sync(full, v, c0), v1 = __shfl_sync(full, v, c0 + 1);
+        const float v2 = __shfl_sync(full, v, c0 + 2), v3 = __shfl_sync(full, v, c0 + 3);
+        if (valid && k == 0) out[agent] = ((v0 + v1) + v2) + v3;
     }
 }
 
@@ -306,12 +402,15 @@ extern "C" int tds_offroad_fwd(const tds_map_t* const* maps, int32_t n_maps, con
     TDS_REQUIRE(d_state && d_lenwid && d_out, "offroad: null pointer");
     MapSetDev set;
     if (int e = tds::gather_maps(maps, n_maps, set)) return e;
-    // agents are dealt round-robin to a grid that fills the GPU a few times over (a CTA per agent would spend a
-    // good part of its life being launched)
+    // groups of 8 agents are dealt round-robin to the warps of a grid that holds them all at once for the benchmark's
+    // 65 536 agents (a warp whose corners are all settled is done after a few hundred cycles)
     TDS_REQUIRE((int64_t)B * A <= 2147483647LL, "offroad: too many agents");
-    const int64_t grid = std::min<int64_t>((int64_t)B * A, (int64_t)tds::sm_count() * 64);
-    offroad_fwd_kernel<<<(unsigned)grid, 128, 0, (cudaStream_t)stream>>>(
-        set, d_env_map, d_state, d_lenwid, d_present, B, A, threshold, d_out, d_face);
+    const int64_t groups = ((int64_t)B * A + 7) / 8;
+    const int64_t grid = std::min<int64_t>((groups + 7) / 8, (int64_t)tds::sm_count() * 16);
+    bool triage = true;
+    if (const char* e = getenv("TDS_OFFROAD_TRIAGE")) triage = atoi(e) != 0;      // test hook: search every corner
+    offroad_fwd_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(
+        set, d_env_map, d_state, d_lenwid, d_present, B, A, threshold, triage, d_out, d_face);
     TDS_LAUNCH_OK();
     return TDS_OK;
 }
@@ -329,5 +428,17 @@ extern "C" int tds_offroad_bwd(const tds_map_t* const* maps, int32_t n_maps, con
     offroad_bwd_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
         set, d_env_map, d_state, d_lenwid, d_present, B, A, threshold, d_face, d_grad_out, d_grad_state, d_grad_lenwid);
     TDS_LAUNCH_OK();
+    return TDS_OK;
+}
+
+int tds::offroad_bound_build(const MapDev& d, uint8_t* obound) {
+    const int64_t n = (int64_t)d.bgx * d.bgy;
+    if (d.nf == 0) {                             // nothing to bound: every corner takes the search, which returns at once
+        TDS_CUDA_OK(cudaMemset(obound, kBoundUnknown, (size_t)n));
+        return TDS_OK;
+    }
+    offroad_bound_kernel<<<(unsigned)((n + 255) / 256), 256>>>(d, obound);
+    TDS_LAUNCH_OK();
+    TDS_CUDA_OK(cudaStreamSynchronize(0));
     return TDS_OK;
 }

@@ -40,7 +40,17 @@ struct MapDev {
                                     // cell the faces are sorted by decreasing area (a containing face is found early)
     float ox0, oy0, ocs, oinv;
     int32_t ogx, ogy, nf;
+    // ---- offroad distance bound: one byte per subcell of a fine grid over the map's bounding box (1 m margin),
+    // row-major.  Code q < 255: every point of the subcell is within q / kBoundPerMetre metres of the road mesh by the
+    // reference's own fp32 distance (offroad.cu, offroad_bound_kernel); 255: unknown.  Subcells are 0.25 m (a power of
+    // two, so the lookup is exact), coarser for maps too large for 16 M subcells.
+    const uint8_t* obound;
+    float bx0, by0, bcs, binv;
+    int32_t bgx, bgy;
 };
+
+constexpr int kBoundPerMetre = 64;  // bound codes are multiples of 1/64 m: (q/64)^2 <= thr is exact as q*q <= thr*4096
+constexpr int kBoundUnknown = 255;
 
 struct MapSetDev {
     MapDev m[TDS_MAX_MAPS];
@@ -51,7 +61,7 @@ struct MapSetDev {
 struct tds_map {
     tds::MapDev dev;
     tds_map_info_t info;
-    void* allocations[10];
+    void* allocations[11];
     int device;
 };
 
@@ -60,4 +70,6 @@ int gather_maps(const tds_map_t* const* maps, int32_t n_maps, MapSetDev& out);
 // coverage patterns of sliver quads (tds_quad_table.h) on the current device: built and uploaded by the first
 // tds_map_create on that device (never inside a raster call, which may be under CUDA-graph capture); NULL before that
 const void* quad_table_device();
+// fills d.obound (d.bgx * d.bgy bytes, device) from the offroad grid of d; synchronous (offroad.cu)
+int offroad_bound_build(const MapDev& d, uint8_t* obound);
 }
