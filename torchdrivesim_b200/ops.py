@@ -1,7 +1,14 @@
-"""Functional ops over libtds_b200.so with autograd wiring (kinematics, discs collision, offroad).
+"""Functional ops over libtds_b200.so with autograd wiring (kinematics, collisions, offroad, raster, observations).
 
 Every function takes CUDA tensors in the reference's layouts and launches on the current torch
 stream.  Nothing here has a CPU implementation; `_lib.ptr` raises on CPU tensors.
+
+The differentiable kernels (kinematic step, pairwise and all-pairs collision, agent boxes, offroad) are launched by one
+private launcher per entry point (`_kinematic_fwd` ... `_offroad_bwd`).  The autograd Functions and `out=` paths here,
+the custom operators of torch_ops.py and `FusedRollout` all call them.  A launcher checks that the shapes of its inputs
+agree before it touches the library, converts them with the `_lib.as_*` helpers (an input already in the kernel's dtype
+and contiguous is passed through without a copy, which CUDA-graph capture relies on), allocates the outputs it is not
+given and launches on the current stream.
 """
 import ctypes
 import math
@@ -23,42 +30,62 @@ def kinematic_params(dt: float = 0.1, max_acceleration: float = 5.0, max_steerin
 
 
 # ------------------------------------------------------------------------------------ kinematics
+def _check_out(out: torch.Tensor, shape, what: str) -> None:
+    if out.dtype != torch.float32 or not out.is_contiguous() or tuple(out.shape) != tuple(shape):
+        raise _lib.TdsError(f"{what}: `out` must be a contiguous float32 tensor of shape {list(shape)}")
+
+
+def _kinematic_inputs(state, action, lr, model):
+    adim = action.shape[-1]
+    if adim not in (2, 4):
+        raise _lib.TdsError("kinematic_step: the action must have 2 or 4 values per agent")
+    s = _lib.as_f32(state).reshape(-1, 4)
+    a = _lib.as_f32(action).reshape(-1, adim)
+    l = None if lr is None else _lib.as_f32(lr).reshape(-1)
+    m = None if model is None else _lib.as_i32(model).reshape(-1)
+    n = s.shape[0]
+    if a.shape[0] != n or (l is not None and l.shape[0] != n) or (m is not None and m.shape[0] != n):
+        raise _lib.TdsError("kinematic_step: state, action, lr and model must agree on the batch shape")
+    return s, a, l, m
+
+
+def _kinematic_fwd(state, action, lr, model, uniform_model, params, out=None):
+    """-> the new state, written into `out` when given (which may alias `state`)."""
+    s, a, l, m = _kinematic_inputs(state, action, lr, model)
+    if out is None:
+        out = torch.empty(state.shape, dtype=torch.float32, device=s.device)
+    else:
+        _check_out(out, state.shape, "kinematic_step")
+    _lib.check(_lib.load().tds_kinematic_step_fwd(_lib.ptr(s), _lib.ptr(a), a.shape[1], _lib.ptr(l), _lib.ptr(m), uniform_model,
+                                                  s.shape[0], ctypes.byref(params), _lib.ptr(out), _lib.stream_ptr(s.device)))
+    return out
+
+
+def _kinematic_bwd(state, action, lr, model, uniform_model, params, grad, out=None):
+    """-> (d state, d action, d lr); `out` holds the three buffers, None for a gradient that is not wanted."""
+    s, a, l, m = _kinematic_inputs(state, action, lr, model)
+    g = _lib.as_f32(grad)
+    if out is None:
+        out = (torch.empty(state.shape, dtype=torch.float32, device=s.device),
+               torch.empty(action.shape, dtype=torch.float32, device=s.device),
+               None if lr is None else torch.empty(lr.shape, dtype=torch.float32, device=s.device))
+    gs, ga, gl = out
+    _lib.check(_lib.load().tds_kinematic_step_bwd(_lib.ptr(s), _lib.ptr(a), a.shape[1], _lib.ptr(l), _lib.ptr(m), uniform_model,
+                                                  s.shape[0], ctypes.byref(params), _lib.ptr(g), _lib.ptr(gs), _lib.ptr(ga),
+                                                  _lib.ptr(gl), _lib.stream_ptr(s.device)))
+    return out
+
+
 class _KinematicStep(torch.autograd.Function):
     @staticmethod
     def forward(ctx, state, action, lr, model, uniform_model, params):
-        lib = _lib.load()
-        shape = state.shape
-        s = _lib.as_f32(state).reshape(-1, 4)
-        adim = action.shape[-1]
-        if adim not in (2, 4):
-            raise _lib.TdsError("kinematic_step: the action must have 2 or 4 values per agent")
-        a = _lib.as_f32(action).reshape(-1, adim)
-        l = None if lr is None else _lib.as_f32(lr).reshape(-1)
-        m = None if model is None else _lib.as_i32(model).reshape(-1)
-        n = s.shape[0]
-        if a.shape[0] != n or (l is not None and l.shape[0] != n) or (m is not None and m.shape[0] != n):
-            raise _lib.TdsError("kinematic_step: state, action, lr and model must agree on the batch shape")
-        out = torch.empty_like(s)
-        _lib.check(lib.tds_kinematic_step_fwd(_lib.ptr(s), _lib.ptr(a), adim, _lib.ptr(l), _lib.ptr(m), uniform_model, n,
-                                              ctypes.byref(params), _lib.ptr(out), _lib.stream_ptr(s.device)))
-        ctx.save_for_backward(s, a, l, m)
-        ctx.meta = (uniform_model, params, shape, action.shape, None if lr is None else lr.shape)
-        return out.reshape(shape)
+        ctx.save_for_backward(state, action, lr, model)
+        ctx.meta = (uniform_model, params)
+        return _kinematic_fwd(state, action, lr, model, uniform_model, params)
 
     @staticmethod
     def backward(ctx, grad_out):
-        lib = _lib.load()
-        s, a, l, m = ctx.saved_tensors
-        uniform_model, params, sshape, ashape, lshape = ctx.meta
-        g = _lib.as_f32(grad_out).reshape(-1, 4)
-        n = s.shape[0]
-        gs = torch.empty_like(s)
-        ga = torch.empty_like(a)
-        gl = None if l is None else torch.empty_like(l)
-        _lib.check(lib.tds_kinematic_step_bwd(_lib.ptr(s), _lib.ptr(a), a.shape[-1], _lib.ptr(l), _lib.ptr(m), uniform_model, n,
-                                              ctypes.byref(params), _lib.ptr(g), _lib.ptr(gs), _lib.ptr(ga), _lib.ptr(gl),
-                                              _lib.stream_ptr(s.device)))
-        return gs.reshape(sshape), ga.reshape(ashape), (None if gl is None else gl.reshape(lshape)), None, None, None
+        return (*_kinematic_bwd(*ctx.saved_tensors, *ctx.meta, grad_out), None, None, None)
 
 
 def kinematic_step(state: torch.Tensor, action: torch.Tensor, lr: Optional[torch.Tensor],
@@ -69,129 +96,153 @@ def kinematic_step(state: torch.Tensor, action: torch.Tensor, lr: Optional[torch
     params = params or kinematic_params()
     if out is None:
         return _KinematicStep.apply(state, action, lr, model, uniform_model, params)
-    if out.dtype != torch.float32 or not out.is_contiguous() or out.shape != state.shape:
-        raise _lib.TdsError("kinematic_step: `out` must be a contiguous float32 tensor of the state's shape")
-    lib = _lib.load()
-    s = _lib.as_f32(state).reshape(-1, 4)
-    adim = action.shape[-1]
-    a = _lib.as_f32(action).reshape(-1, adim)
-    l = None if lr is None else _lib.as_f32(lr).reshape(-1)
-    m = None if model is None else _lib.as_i32(model).reshape(-1)
-    _lib.check(lib.tds_kinematic_step_fwd(_lib.ptr(s), _lib.ptr(a), adim, _lib.ptr(l), _lib.ptr(m), uniform_model, s.shape[0],
-                                          ctypes.byref(params), _lib.ptr(out), _lib.stream_ptr(s.device)))
-    return out
+    return _kinematic_fwd(state, action, lr, model, uniform_model, params, out)
 
 
 # ------------------------------------------------------------------------------------ collisions
+def _pairwise_inputs(box1, box2):
+    if box1.shape != box2.shape or box1.shape[-1] != 5:
+        raise _lib.TdsError("collision_pairwise: boxes must have identical shape [...,5]")
+    return _lib.as_f32(box1), _lib.as_f32(box2)
+
+
+def _pairwise_fwd(box1, box2, metric):
+    b1, b2 = _pairwise_inputs(box1, box2)
+    out = torch.empty(b1.shape[:-1], dtype=torch.float32, device=b1.device)
+    _lib.check(_lib.load().tds_collision_pairwise_fwd(_lib.ptr(b1), _lib.ptr(b2), out.numel(), metric, _lib.ptr(out),
+                                                      _lib.stream_ptr(b1.device)))
+    return out
+
+
+def _pairwise_bwd(box1, box2, metric, grad):
+    b1, b2 = _pairwise_inputs(box1, box2)
+    g = _lib.as_f32(grad)
+    g1, g2 = torch.empty_like(b1), torch.empty_like(b2)
+    _lib.check(_lib.load().tds_collision_pairwise_bwd(_lib.ptr(b1), _lib.ptr(b2), b1.numel() // 5, metric, _lib.ptr(g),
+                                                      _lib.ptr(g1), _lib.ptr(g2), _lib.stream_ptr(b1.device)))
+    return g1, g2
+
+
 class _Pairwise(torch.autograd.Function):
     @staticmethod
     def forward(ctx, box1, box2, metric):
-        lib = _lib.load()
-        b1 = _lib.as_f32(box1).reshape(-1, 5)
-        b2 = _lib.as_f32(box2).reshape(-1, 5)
-        out = torch.empty(b1.shape[0], dtype=torch.float32, device=b1.device)
-        _lib.check(lib.tds_collision_pairwise_fwd(_lib.ptr(b1), _lib.ptr(b2), b1.shape[0], metric,
-                                                  _lib.ptr(out), _lib.stream_ptr(b1.device)))
-        ctx.save_for_backward(b1, b2)
-        ctx.meta = (box1.shape, box2.shape, metric)
-        return out.reshape(box1.shape[:-1])
+        ctx.save_for_backward(box1, box2)
+        ctx.metric = metric
+        return _pairwise_fwd(box1, box2, metric)
 
     @staticmethod
     def backward(ctx, grad_out):
-        lib = _lib.load()
-        b1, b2 = ctx.saved_tensors
-        g = _lib.as_f32(grad_out).reshape(-1)
-        g1, g2 = torch.empty_like(b1), torch.empty_like(b2)
-        _lib.check(lib.tds_collision_pairwise_bwd(_lib.ptr(b1), _lib.ptr(b2), b1.shape[0], ctx.meta[2], _lib.ptr(g),
-                                                  _lib.ptr(g1), _lib.ptr(g2), _lib.stream_ptr(b1.device)))
-        return g1.reshape(ctx.meta[0]), g2.reshape(ctx.meta[1]), None
+        return (*_pairwise_bwd(*ctx.saved_tensors, ctx.metric, grad_out), None)
 
 
 def collision_pairwise(box1: torch.Tensor, box2: torch.Tensor, metric: int = _lib.METRIC_DISCS) -> torch.Tensor:
     """Element-wise overlap of box1[...,5] and box2[...,5] (same shape) -> [...], differentiable."""
-    if box1.shape != box2.shape or box1.shape[-1] != 5:
-        raise _lib.TdsError("collision_pairwise: boxes must have identical shape [...,5]")
     return _Pairwise.apply(box1, box2, metric)
 
 
-class _AllPairs(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, ego_box, all_box, mask, metric, ego_is_prefix):
-        lib = _lib.load()
-        e = _lib.as_f32(ego_box)
-        a = _lib.as_f32(all_box)
-        m = _lib.as_u8(mask)
-        B, A, N = e.shape[0], e.shape[1], a.shape[1]
-        out = torch.empty(B, A, dtype=torch.float32, device=e.device)       # the kernel writes every row
-        arg = torch.empty(B, A, dtype=torch.int32, device=e.device)
-        _lib.check(lib.tds_collision_allpairs_fwd(_lib.ptr(e), _lib.ptr(a), _lib.ptr(m), B, A, N, metric,
-                                                  1 if ego_is_prefix else 0, _lib.ptr(out), _lib.ptr(arg),
-                                                  _lib.stream_ptr(e.device)))
-        ctx.save_for_backward(e, a, m, arg)
-        ctx.meta = (metric, 1 if ego_is_prefix else 0)
-        return out
-
-    @staticmethod
-    def backward(ctx, grad_out):
-        lib = _lib.load()
-        e, a, m, arg = ctx.saved_tensors
-        B, A, N = e.shape[0], e.shape[1], a.shape[1]
-        g = _lib.as_f32(grad_out)
-        ge = torch.zeros_like(e)
-        ga = torch.zeros_like(a)
-        _lib.check(lib.tds_collision_allpairs_bwd(_lib.ptr(e), _lib.ptr(a), _lib.ptr(m), B, A, N, ctx.meta[0], ctx.meta[1],
-                                                  _lib.ptr(g), _lib.ptr(arg), _lib.ptr(ge), _lib.ptr(ga),
-                                                  _lib.stream_ptr(e.device)))
-        return ge, ga, None, None, None
-
-
-def collision_allpairs(ego_box: torch.Tensor, all_box: torch.Tensor, mask: torch.Tensor,
-                       metric: int = _lib.METRIC_DISCS, ego_is_prefix: bool = True, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Fused Simulator.compute_collision: ego_box [B,A,5], all_box [B,N,5], mask [B,N] -> [B,A], differentiable.
-    `out` (contiguous float32 [B,A]): written directly, no autograd tape."""
+def _allpairs_inputs(ego_box, all_box, mask, metric):
     if ego_box.dim() != 3 or all_box.dim() != 3 or ego_box.shape[-1] != 5 or all_box.shape[-1] != 5:
         raise _lib.TdsError("collision_allpairs: expected ego_box [B,A,5] and all_box [B,N,5]")
     if ego_box.shape[0] != all_box.shape[0] or tuple(mask.shape) != tuple(all_box.shape[:2]):
         raise _lib.TdsError("collision_allpairs: batch / mask shape mismatch")
     if metric not in (_lib.METRIC_DISCS, _lib.METRIC_IOU):
         raise _lib.TdsError(f"collision_allpairs: unknown metric {metric}")
+    return _lib.as_f32(ego_box), _lib.as_f32(all_box), _lib.as_u8(mask)
+
+
+def _allpairs_fwd(ego_box, all_box, mask, metric, ego_is_prefix, out=None):
+    """-> (overlap [B,A] float32, argmax [B,A] int32); `out` holds the two buffers (argmax None: not written)."""
+    e, a, m = _allpairs_inputs(ego_box, all_box, mask, metric)
+    B, A, N = e.shape[0], e.shape[1], a.shape[1]
+    if out is None:          # the kernel writes every row
+        out = (torch.empty(B, A, dtype=torch.float32, device=e.device), torch.empty(B, A, dtype=torch.int32, device=e.device))
+    else:
+        _check_out(out[0], (B, A), "collision_allpairs")
+    _lib.check(_lib.load().tds_collision_allpairs_fwd(_lib.ptr(e), _lib.ptr(a), _lib.ptr(m), B, A, N, metric,
+                                                      1 if ego_is_prefix else 0, _lib.ptr(out[0]), _lib.ptr(out[1]),
+                                                      _lib.stream_ptr(e.device)))
+    return out
+
+
+def _allpairs_bwd(ego_box, all_box, mask, metric, ego_is_prefix, argmax, grad, out=None):
+    """-> (d ego_box, d all_box); `out` holds the two buffers.  The kernel accumulates into d all_box, which is zeroed
+    here first."""
+    e, a, m = _allpairs_inputs(ego_box, all_box, mask, metric)
+    B, A, N = e.shape[0], e.shape[1], a.shape[1]
+    if tuple(argmax.shape) != (B, A):
+        raise _lib.TdsError("collision_allpairs: argmax must be [B,A]")
+    g = _lib.as_f32(grad)
+    ge, ga = (torch.zeros_like(e), torch.zeros_like(a)) if out is None else (out[0], out[1].zero_())
+    _lib.check(_lib.load().tds_collision_allpairs_bwd(_lib.ptr(e), _lib.ptr(a), _lib.ptr(m), B, A, N, metric,
+                                                      1 if ego_is_prefix else 0, _lib.ptr(g),
+                                                      _lib.ptr(_lib.as_i32(argmax)), _lib.ptr(ge), _lib.ptr(ga),
+                                                      _lib.stream_ptr(e.device)))
+    return ge, ga
+
+
+class _AllPairs(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, ego_box, all_box, mask, metric, ego_is_prefix):
+        out, arg = _allpairs_fwd(ego_box, all_box, mask, metric, ego_is_prefix)
+        ctx.save_for_backward(ego_box, all_box, mask, arg)
+        ctx.meta = (metric, ego_is_prefix)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        ego_box, all_box, mask, arg = ctx.saved_tensors
+        return (*_allpairs_bwd(ego_box, all_box, mask, *ctx.meta, arg, grad_out), None, None, None)
+
+
+def collision_allpairs(ego_box: torch.Tensor, all_box: torch.Tensor, mask: torch.Tensor,
+                       metric: int = _lib.METRIC_DISCS, ego_is_prefix: bool = True, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Fused Simulator.compute_collision: ego_box [B,A,5], all_box [B,N,5], mask [B,N] -> [B,A], differentiable.
+    `out` (contiguous float32 [B,A]): written directly, no autograd tape."""
     if out is None:
         return _AllPairs.apply(ego_box, all_box, mask, metric, ego_is_prefix)
-    e, a, m = _lib.as_f32(ego_box), _lib.as_f32(all_box), _lib.as_u8(mask)
-    if out.dtype != torch.float32 or not out.is_contiguous() or tuple(out.shape) != tuple(e.shape[:2]):
-        raise _lib.TdsError("collision_allpairs: `out` must be a contiguous float32 [B,A] tensor")
-    _lib.check(_lib.load().tds_collision_allpairs_fwd(_lib.ptr(e), _lib.ptr(a), _lib.ptr(m), e.shape[0], e.shape[1], a.shape[1], metric,
-                                                      1 if ego_is_prefix else 0, _lib.ptr(out), None, _lib.stream_ptr(e.device)))
+    return _allpairs_fwd(ego_box, all_box, mask, metric, ego_is_prefix, (out, None))[0]
+
+
+def _agent_boxes(state, size=None, out=None):
+    """state [...,4], size [...,2+] -> boxes [...,5]; without `size`: the camera of every agent, (xy [...,2],
+    (sin psi, cos psi) [...,2]).  `out`: the boxes, or the (xy, sincos) pair."""
+    if state.shape[-1] != 4 or (size is not None and (size.shape[-1] < 2 or state.shape[:-1] != size.shape[:-1])):
+        raise _lib.TdsError("agent_boxes: expected state [...,4] and size [...,2]")
+    s = _lib.as_f32(state)
+    z = None if size is None else _lib.as_f32(size[..., :2])
+    if out is None:
+        f32 = dict(dtype=torch.float32, device=s.device)
+        out = (torch.empty(s.shape[:-1] + (5,), **f32) if size is not None else
+               (torch.empty(s.shape[:-1] + (2,), **f32), torch.empty(s.shape[:-1] + (2,), **f32)))
+    box, (xy, sc) = (out, (None, None)) if size is not None else (None, out)
+    _lib.check(_lib.load().tds_agent_boxes(_lib.ptr(s), _lib.ptr(z), s.numel() // 4, _lib.ptr(box), _lib.ptr(sc), _lib.ptr(xy),
+                                           _lib.stream_ptr(s.device)))
     return out
+
+
+def _agent_boxes_grad(g, size_cols: int):
+    """d boxes [...,5] -> (d state [...,4], d size [...,size_cols])."""
+    gs = torch.cat([g[..., 0:2], g[..., 4:5], torch.zeros_like(g[..., 0:1])], dim=-1)
+    gz = g[..., 2:4]
+    if size_cols > 2:
+        gz = torch.cat([gz, g.new_zeros(gz.shape[:-1] + (size_cols - 2,))], dim=-1)
+    return gs, gz
 
 
 class _AgentBoxes(torch.autograd.Function):
     @staticmethod
     def forward(ctx, state, size):
-        lib = _lib.load()
-        s = _lib.as_f32(state)
-        z = _lib.as_f32(size[..., :2])
-        n = s[..., 0].numel()
-        box = torch.empty(s.shape[:-1] + (5,), dtype=torch.float32, device=s.device)
-        _lib.check(lib.tds_agent_boxes(_lib.ptr(s), _lib.ptr(z), n, _lib.ptr(box), None, None, _lib.stream_ptr(s.device)))
-        ctx.meta = (state.shape, size.shape)
-        return box
+        ctx.size_cols = size.shape[-1]
+        return _agent_boxes(state, size)
 
     @staticmethod
     def backward(ctx, g):
-        sshape, zshape = ctx.meta
-        gs = torch.cat([g[..., 0:2], g[..., 4:5], torch.zeros_like(g[..., 0:1])], dim=-1)
-        gz = g[..., 2:4]
-        if zshape[-1] > 2:
-            gz = torch.cat([gz, torch.zeros(gz.shape[:-1] + (zshape[-1] - 2,), dtype=gz.dtype, device=gz.device)], dim=-1)
-        return gs.reshape(sshape), gz.reshape(zshape)
+        return _agent_boxes_grad(g, ctx.size_cols)
 
 
 def agent_boxes(state: torch.Tensor, size: torch.Tensor) -> torch.Tensor:
     """state [...,4] (x, y, psi, v), size [...,2+] (length, width) -> boxes [...,5] (x, y, length, width, psi): the layout of
     compute_collision (simulator.py:1161-1170) in one launch instead of a torch.cat; differentiable."""
-    if state.shape[-1] != 4 or size.shape[-1] < 2 or state.shape[:-1] != size.shape[:-1]:
-        raise _lib.TdsError("agent_boxes: expected state [...,4] and size [...,2]")
     return _AgentBoxes.apply(state, size)
 
 
@@ -199,12 +250,7 @@ def egocentric_cameras(state: torch.Tensor):
     """state [...,4] -> (xy [...,2] contiguous, (sin psi, cos psi) [...,2]): the camera of every agent in one launch, the
     heading evaluated like every other heading of the path (float64, rounded) - render_egocentric, simulator.py:961,
     1017.  Not differentiable."""
-    lib = _lib.load()
-    s = _lib.as_f32(state)
-    xy = torch.empty(s.shape[:-1] + (2,), dtype=torch.float32, device=s.device)
-    sc = torch.empty_like(xy)
-    _lib.check(lib.tds_agent_boxes(_lib.ptr(s), None, s[..., 0].numel(), None, _lib.ptr(sc), _lib.ptr(xy), _lib.stream_ptr(s.device)))
-    return xy, sc
+    return _agent_boxes(state)
 
 
 def heading_sincos(state: torch.Tensor) -> torch.Tensor:
@@ -309,61 +355,67 @@ def infraction_metrics(collision: torch.Tensor, offroad: torch.Tensor, present: 
 
 
 # ------------------------------------------------------------------------------------ offroad
+def _offroad_inputs(state, lenwid, present):
+    if state.dim() != 3 or state.shape[-1] != 4:
+        raise _lib.TdsError("offroad: expected state [B,A,4]")
+    if tuple(lenwid.shape) != (state.shape[0], state.shape[1], 2):
+        raise _lib.TdsError("offroad: expected lenwid [B,A,2] or [B,2]")
+    if present is not None and tuple(present.shape) != tuple(state.shape[:2]):
+        raise _lib.TdsError("offroad: expected present [B,A]")
+    return _lib.as_f32(state), _lib.as_f32(lenwid), None if present is None else _lib.as_u8(present)
+
+
+def _offroad_fwd(state, lenwid, present, mapset, threshold, out=None):
+    """-> (offroad [B,A] float32, face [B,A,4] int32: the face each corner was measured to, -1 for none); `out` holds
+    the two buffers (face None: not written)."""
+    s, lw, p = _offroad_inputs(state, lenwid, present)
+    B, A = s.shape[0], s.shape[1]
+    if out is None:          # the kernel writes every agent
+        out = (torch.empty(B, A, dtype=torch.float32, device=s.device), torch.empty(B, A, 4, dtype=torch.int32, device=s.device))
+    else:
+        _check_out(out[0], (B, A), "offroad")
+    handles, n_maps = mapset.handles(s.device)
+    _lib.check(_lib.load().tds_offroad_fwd(handles, n_maps, _lib.ptr(mapset.env_map_on(s.device)), _lib.ptr(s), _lib.ptr(lw),
+                                           _lib.ptr(p), B, A, float(threshold), _lib.ptr(out[0]), _lib.ptr(out[1]),
+                                           _lib.stream_ptr(s.device)))
+    return out
+
+
+def _offroad_bwd(state, lenwid, present, mapset, threshold, face, grad, out=None):
+    """-> (d state, d lenwid); `out` holds the two buffers, None for a gradient that is not wanted."""
+    s, lw, p = _offroad_inputs(state, lenwid, present)
+    g = _lib.as_f32(grad)
+    gs, gl = (torch.zeros_like(s), torch.zeros_like(lw)) if out is None else out
+    handles, n_maps = mapset.handles(s.device)
+    _lib.check(_lib.load().tds_offroad_bwd(handles, n_maps, _lib.ptr(mapset.env_map_on(s.device)), _lib.ptr(s), _lib.ptr(lw),
+                                           _lib.ptr(p), s.shape[0], s.shape[1], float(threshold), _lib.ptr(face), _lib.ptr(g),
+                                           _lib.ptr(gs), _lib.ptr(gl), _lib.stream_ptr(s.device)))
+    return gs, gl
+
+
 class _Offroad(torch.autograd.Function):
     @staticmethod
     def forward(ctx, state, lenwid, present, mapset, threshold):
-        lib = _lib.load()
-        s = _lib.as_f32(state)
-        lw = _lib.as_f32(lenwid)
-        p = None if present is None else _lib.as_u8(present)
-        B, A = s.shape[0], s.shape[1]
-        handles, n_maps = mapset.handles(s.device)
-        env_map = mapset.env_map_on(s.device)
-        out = torch.empty(B, A, dtype=torch.float32, device=s.device)       # the kernel writes every agent
-        face = torch.empty(B, A, 4, dtype=torch.int32, device=s.device)
-        _lib.check(lib.tds_offroad_fwd(handles, n_maps, _lib.ptr(env_map), _lib.ptr(s), _lib.ptr(lw), _lib.ptr(p), B, A,
-                                       float(threshold), _lib.ptr(out), _lib.ptr(face), _lib.stream_ptr(s.device)))
-        ctx.save_for_backward(s, lw, p, face)
-        ctx.meta = (mapset, float(threshold), state.shape, lenwid.shape)
+        out, face = _offroad_fwd(state, lenwid, present, mapset, threshold)
+        ctx.save_for_backward(state, lenwid, present, face)
+        ctx.meta = (mapset, threshold)
         return out
 
     @staticmethod
     def backward(ctx, grad_out):
-        lib = _lib.load()
-        s, lw, p, face = ctx.saved_tensors
-        mapset, threshold, sshape, lshape = ctx.meta
-        B, A = s.shape[0], s.shape[1]
-        handles, n_maps = mapset.handles(s.device)
-        env_map = mapset.env_map_on(s.device)
-        g = _lib.as_f32(grad_out)
-        gs = torch.zeros_like(s)
-        gl = torch.zeros_like(lw)
-        _lib.check(lib.tds_offroad_bwd(handles, n_maps, _lib.ptr(env_map), _lib.ptr(s), _lib.ptr(lw), _lib.ptr(p), B, A,
-                                       threshold, _lib.ptr(face), _lib.ptr(g), _lib.ptr(gs), _lib.ptr(gl),
-                                       _lib.stream_ptr(s.device)))
-        return gs.reshape(sshape), gl.reshape(lshape), None, None, None
+        state, lenwid, present, face = ctx.saved_tensors
+        return (*_offroad_bwd(state, lenwid, present, *ctx.meta, face, grad_out), None, None, None)
 
 
 def offroad(state: torch.Tensor, lenwid: torch.Tensor, mapset: MapSet, threshold: float = 0.0,
             present: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """state [B,A,4], lenwid [B,A,2] -> [B,A] sum over corners of thresholded squared distance to the map.
-    `out` (contiguous float32 [B,A]): written directly, no autograd tape."""
-    if state.dim() != 3 or state.shape[-1] != 4:
-        raise _lib.TdsError("offroad: expected state [B,A,4]")
-    if lenwid.dim() == 2:
+    """state [B,A,4], lenwid [B,A,2] or [B,2], present [B,A] -> [B,A] sum over corners of thresholded squared distance
+    to the map.  `out` (contiguous float32 [B,A]): written directly, no autograd tape."""
+    if lenwid.dim() == 2 and state.dim() == 3:
         lenwid = lenwid.unsqueeze(-2).expand(lenwid.shape[0], state.shape[1], lenwid.shape[1])
-    if tuple(lenwid.shape) != (state.shape[0], state.shape[1], 2):
-        raise _lib.TdsError("offroad: expected lenwid [B,A,2] or [B,2]")
     if out is None:
         return _Offroad.apply(state, lenwid, present, mapset, threshold)
-    s, lw = _lib.as_f32(state), _lib.as_f32(lenwid)
-    p = None if present is None else _lib.as_u8(present)
-    if out.dtype != torch.float32 or not out.is_contiguous() or tuple(out.shape) != tuple(s.shape[:2]):
-        raise _lib.TdsError("offroad: `out` must be a contiguous float32 [B,A] tensor")
-    handles, n_maps = mapset.handles(s.device)
-    _lib.check(_lib.load().tds_offroad_fwd(handles, n_maps, _lib.ptr(mapset.env_map_on(s.device)), _lib.ptr(s), _lib.ptr(lw), _lib.ptr(p),
-                                           s.shape[0], s.shape[1], float(threshold), _lib.ptr(out), None, _lib.stream_ptr(s.device)))
-    return out
+    return _offroad_fwd(state, lenwid, present, mapset, threshold, (out, None))[0]
 
 
 # ------------------------------------------------------------------------------------ raster

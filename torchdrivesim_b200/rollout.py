@@ -3,8 +3,10 @@ collision loss", examples/imitation_learning.py:279-335 in the reference).
 
 Through autograd a T-step rollout is ~30 small launches per step: every `Simulator.step` / `compute_collision` /
 `compute_offroad` is a custom autograd Function around a 5 us kernel, plus torch glue (cat, sum, pow, mean) and their
-backward nodes - the GPU idles between launches.  `FusedRollout` issues the same kernels through the C ABI in a fixed
-order, forward and backward, into static buffers and records the sequence once:
+backward nodes - the GPU idles between launches.  `FusedRollout` issues the same kernels through the same launchers of
+ops.py in a fixed order, forward and backward, into static buffers and records the sequence once.  Its inputs are kept
+in the kernels' dtypes (the present mask as bool), so the launchers pass them through without a copy; only the loss
+and the gradient merge call the C ABI directly:
 
     forward,  t = 0..T-1:  kinematic step -> boxes -> all-pairs collision -> offroad -> loss accumulation
     backward, t = T-1..0:  offroad backward, collision backward -> merge with the gradient from step t+1 and the
@@ -15,7 +17,6 @@ order, forward and backward, into static buffers and records the sequence once:
 The gradients are those the eager path (`ops.*` autograd Functions) produces; tests/test_gpu_rollout.py checks them
 against it and against the oracle's torch-autograd restatement.
 """
-import ctypes
 from typing import Optional, Tuple
 
 import torch
@@ -45,7 +46,7 @@ class FusedRollout:
         self.state[0].copy_(_lib.as_f32(state0))
         self.size = _lib.as_f32(agent_size[..., :2]).clone()
         self.lr = _lib.as_f32(lr).clone()
-        self.present = _lib.as_u8(present_mask).clone()
+        self.present = (present_mask.detach() != 0).contiguous()     # bool: the launchers view it as uint8, no copy
         self.model = None if model is None else _lib.as_i32(model).clone()
         self.uniform_model = int(uniform_model)
         self.params = ops.kinematic_params(dt=dt, left_handed=left_handed)
@@ -71,8 +72,6 @@ class FusedRollout:
         n_agents = B * A
         self._scale = torch.tensor([self.w[0], self.w[1], 0.0 if self.target is None else self.w[2] / (2 * n_agents)],
                                    dtype=torch.float64, device=dev)
-        self.handles, self.n_maps = self.mapset.handles(dev)
-        self.env_map = self.mapset.env_map_on(dev)
         # warm up on a side stream (lazily built map handles, allocator), then capture
         s = torch.cuda.Stream(device=dev)
         s.wait_stream(torch.cuda.current_stream(dev))
@@ -95,32 +94,27 @@ class FusedRollout:
         wc, wo, wt = self.w
         # the target term is w_t * mean over (agents, xy) of the squared error = w_t / (2 n) * sum |xy - target|^2
         wt_grad = 0.0 if self.target is None else wt / n
+        kin = (self.lr, self.model, self.uniform_model, self.params)
+        off = (self.size, self.present, self.mapset, self.threshold)
         self.acc.zero_()
         for t in range(T):
             s0, s1 = self.state[t], self.state[t + 1]
-            _lib.check(lib.tds_kinematic_step_fwd(p(s0), p(self.actions[t]), 2, p(self.lr), p(self.model), self.uniform_model, n,
-                                                  ctypes.byref(self.params), p(s1), st))
-            _lib.check(lib.tds_agent_boxes(p(s1), p(self.size), n, p(self.box[t]), None, None, st))
-            _lib.check(lib.tds_collision_allpairs_fwd(p(self.box[t]), p(self.box[t]), p(self.present), B, A, A, self.metric, 1,
-                                                      p(self.collision), p(self.argmax[t]), st))
-            _lib.check(lib.tds_offroad_fwd(self.handles, self.n_maps, p(self.env_map), p(s1), p(self.size), p(self.present), B, A,
-                                           self.threshold, p(self.offroad), p(self.face[t]), st))
+            ops._kinematic_fwd(s0, self.actions[t], *kin, out=s1)
+            ops._agent_boxes(s1, self.size, out=self.box[t])
+            ops._allpairs_fwd(self.box[t], self.box[t], self.present, self.metric, True, out=(self.collision, self.argmax[t]))
+            ops._offroad_fwd(s1, *off, out=(self.offroad, self.face[t]))
             _lib.check(lib.tds_rollout_loss(p(self.collision), p(self.offroad), p(s1), p(self.target), n, p(self.acc), st))
         self.loss.copy_((self.acc * self._scale).sum())
         g_next = None
         for t in range(T - 1, -1, -1):
             s0, s1 = self.state[t], self.state[t + 1]
-            _lib.check(lib.tds_offroad_bwd(self.handles, self.n_maps, p(self.env_map), p(s1), p(self.size), p(self.present), B, A,
-                                           self.threshold, p(self.face[t]), p(self.ones), p(self.g_off), None, st))
-            self.g_all.zero_()
-            _lib.check(lib.tds_collision_allpairs_bwd(p(self.box[t]), p(self.box[t]), p(self.present), B, A, A, self.metric, 1,
-                                                      p(self.ones), p(self.argmax[t]), p(self.g_ego), p(self.g_all), st))
+            ops._offroad_bwd(s1, *off, self.face[t], self.ones, out=(self.g_off, None))
+            ops._allpairs_bwd(self.box[t], self.box[t], self.present, self.metric, True, self.argmax[t], self.ones,
+                              out=(self.g_ego, self.g_all))
             _lib.check(lib.tds_rollout_grad(None if g_next is None else p(g_next), p(self.g_off), p(self.g_ego), p(self.g_all),
                                             p(s1), p(self.target), wo, wc, wt_grad, n, p(self.g_merged), st))
             g_out = self.g_state[t & 1]
-            _lib.check(lib.tds_kinematic_step_bwd(p(s0), p(self.actions[t]), 2, p(self.lr), p(self.model), self.uniform_model, n,
-                                                  ctypes.byref(self.params), p(self.g_merged), p(g_out), p(self.grad_actions[t]),
-                                                  None, st))
+            ops._kinematic_bwd(s0, self.actions[t], *kin, self.g_merged, out=(g_out, self.grad_actions[t], None))
             g_next = g_out
         self.grad_state0 = g_next
 

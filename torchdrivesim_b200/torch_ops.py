@@ -9,37 +9,26 @@ not a tensor.
     torch.ops.tds_b200.collision_allpairs(ego_box, all_box, mask, metric, ego_is_prefix) -> (loss, argmax)
     torch.ops.tds_b200.agent_boxes(state, size) -> boxes
 
+This module holds the registrations only: every operator body calls the launcher of ops.py that the autograd Functions
+use too, so both check their inputs and launch the kernels the same way.
+
 Reference call sites: kinematic.py:462-523, infractions.py:503-545 / 307-324, simulator.py:1161-1194.
 """
-import ctypes
 from typing import Optional, Tuple
 
 import torch
 from torch import Tensor
 
-from . import _lib, ops
+from . import ops
 
 _NS = "tds_b200"
-
-
-def _params(dt: float, left_handed: bool):
-    return ops.kinematic_params(dt=dt, left_handed=left_handed)
 
 
 # ------------------------------------------------------------------------------------ kinematic step
 @torch.library.custom_op(f"{_NS}::kinematic_step", mutates_args=())
 def kinematic_step(state: Tensor, action: Tensor, lr: Tensor, model: Optional[Tensor], uniform_model: int, dt: float,
                    left_handed: bool) -> Tensor:
-    lib = _lib.load()
-    s = _lib.as_f32(state).reshape(-1, 4)
-    a = _lib.as_f32(action).reshape(-1, action.shape[-1])
-    l = _lib.as_f32(lr).reshape(-1)
-    m = None if model is None else _lib.as_i32(model).reshape(-1)
-    out = torch.empty_like(s)
-    p = _params(dt, left_handed)
-    _lib.check(lib.tds_kinematic_step_fwd(_lib.ptr(s), _lib.ptr(a), a.shape[-1], _lib.ptr(l), _lib.ptr(m), uniform_model, s.shape[0],
-                                          ctypes.byref(p), _lib.ptr(out), _lib.stream_ptr(s.device)))
-    return out.reshape(state.shape)
+    return ops._kinematic_fwd(state, action, lr, model, uniform_model, ops.kinematic_params(dt=dt, left_handed=left_handed))
 
 
 @kinematic_step.register_fake
@@ -50,17 +39,8 @@ def _(state, action, lr, model, uniform_model, dt, left_handed):
 @torch.library.custom_op(f"{_NS}::kinematic_step_backward", mutates_args=())
 def kinematic_step_backward(grad_out: Tensor, state: Tensor, action: Tensor, lr: Tensor, model: Optional[Tensor], uniform_model: int,
                             dt: float, left_handed: bool) -> Tuple[Tensor, Tensor, Tensor]:
-    lib = _lib.load()
-    s = _lib.as_f32(state).reshape(-1, 4)
-    a = _lib.as_f32(action).reshape(-1, action.shape[-1])
-    l = _lib.as_f32(lr).reshape(-1)
-    m = None if model is None else _lib.as_i32(model).reshape(-1)
-    g = _lib.as_f32(grad_out).reshape(-1, 4)
-    gs, ga, gl = torch.empty_like(s), torch.empty_like(a), torch.empty_like(l)
-    p = _params(dt, left_handed)
-    _lib.check(lib.tds_kinematic_step_bwd(_lib.ptr(s), _lib.ptr(a), a.shape[-1], _lib.ptr(l), _lib.ptr(m), uniform_model, s.shape[0],
-                                          ctypes.byref(p), _lib.ptr(g), _lib.ptr(gs), _lib.ptr(ga), _lib.ptr(gl), _lib.stream_ptr(s.device)))
-    return gs.reshape(state.shape), ga.reshape(action.shape), gl.reshape(lr.shape)
+    return ops._kinematic_bwd(state, action, lr, model, uniform_model, ops.kinematic_params(dt=dt, left_handed=left_handed),
+                              grad_out)
 
 
 @kinematic_step_backward.register_fake
@@ -87,11 +67,7 @@ kinematic_step.register_autograd(_kin_backward, setup_context=_kin_setup)
 # ------------------------------------------------------------------------------------ collisions
 @torch.library.custom_op(f"{_NS}::collision_pairwise", mutates_args=())
 def collision_pairwise(box1: Tensor, box2: Tensor, metric: int) -> Tensor:
-    lib = _lib.load()
-    b1, b2 = _lib.as_f32(box1).reshape(-1, 5), _lib.as_f32(box2).reshape(-1, 5)
-    out = torch.empty(b1.shape[0], dtype=torch.float32, device=b1.device)
-    _lib.check(lib.tds_collision_pairwise_fwd(_lib.ptr(b1), _lib.ptr(b2), b1.shape[0], metric, _lib.ptr(out), _lib.stream_ptr(b1.device)))
-    return out.reshape(box1.shape[:-1])
+    return ops._pairwise_fwd(box1, box2, metric)
 
 
 @collision_pairwise.register_fake
@@ -101,13 +77,7 @@ def _(box1, box2, metric):
 
 @torch.library.custom_op(f"{_NS}::collision_pairwise_backward", mutates_args=())
 def collision_pairwise_backward(grad_out: Tensor, box1: Tensor, box2: Tensor, metric: int) -> Tuple[Tensor, Tensor]:
-    lib = _lib.load()
-    b1, b2 = _lib.as_f32(box1).reshape(-1, 5), _lib.as_f32(box2).reshape(-1, 5)
-    g = _lib.as_f32(grad_out).reshape(-1)
-    g1, g2 = torch.empty_like(b1), torch.empty_like(b2)
-    _lib.check(lib.tds_collision_pairwise_bwd(_lib.ptr(b1), _lib.ptr(b2), b1.shape[0], metric, _lib.ptr(g), _lib.ptr(g1), _lib.ptr(g2),
-                                              _lib.stream_ptr(b1.device)))
-    return g1.reshape(box1.shape), g2.reshape(box2.shape)
+    return ops._pairwise_bwd(box1, box2, metric, grad_out)
 
 
 @collision_pairwise_backward.register_fake
@@ -122,14 +92,7 @@ collision_pairwise.register_autograd(
 
 @torch.library.custom_op(f"{_NS}::collision_allpairs", mutates_args=())
 def collision_allpairs(ego_box: Tensor, all_box: Tensor, mask: Tensor, metric: int, ego_is_prefix: bool) -> Tuple[Tensor, Tensor]:
-    lib = _lib.load()
-    e, a, m = _lib.as_f32(ego_box), _lib.as_f32(all_box), _lib.as_u8(mask)
-    B, A, N = e.shape[0], e.shape[1], a.shape[1]
-    out = torch.empty(B, A, dtype=torch.float32, device=e.device)
-    arg = torch.empty(B, A, dtype=torch.int32, device=e.device)
-    _lib.check(lib.tds_collision_allpairs_fwd(_lib.ptr(e), _lib.ptr(a), _lib.ptr(m), B, A, N, metric, 1 if ego_is_prefix else 0,
-                                              _lib.ptr(out), _lib.ptr(arg), _lib.stream_ptr(e.device)))
-    return out, arg
+    return ops._allpairs_fwd(ego_box, all_box, mask, metric, ego_is_prefix)
 
 
 @collision_allpairs.register_fake
@@ -141,14 +104,7 @@ def _(ego_box, all_box, mask, metric, ego_is_prefix):
 @torch.library.custom_op(f"{_NS}::collision_allpairs_backward", mutates_args=())
 def collision_allpairs_backward(grad_out: Tensor, ego_box: Tensor, all_box: Tensor, mask: Tensor, argmax: Tensor, metric: int,
                                 ego_is_prefix: bool) -> Tuple[Tensor, Tensor]:
-    lib = _lib.load()
-    e, a, m = _lib.as_f32(ego_box), _lib.as_f32(all_box), _lib.as_u8(mask)
-    B, A, N = e.shape[0], e.shape[1], a.shape[1]
-    ge, ga = torch.zeros_like(e), torch.zeros_like(a)
-    _lib.check(lib.tds_collision_allpairs_bwd(_lib.ptr(e), _lib.ptr(a), _lib.ptr(m), B, A, N, metric, 1 if ego_is_prefix else 0,
-                                              _lib.ptr(_lib.as_f32(grad_out)), _lib.ptr(argmax.contiguous()), _lib.ptr(ge), _lib.ptr(ga),
-                                              _lib.stream_ptr(e.device)))
-    return ge, ga
+    return ops._allpairs_bwd(ego_box, all_box, mask, metric, ego_is_prefix, argmax, grad_out)
 
 
 @collision_allpairs_backward.register_fake
@@ -175,11 +131,7 @@ collision_allpairs.register_autograd(_ap_backward, setup_context=_ap_setup)
 # ------------------------------------------------------------------------------------ boxes
 @torch.library.custom_op(f"{_NS}::agent_boxes", mutates_args=())
 def agent_boxes(state: Tensor, size: Tensor) -> Tensor:
-    lib = _lib.load()
-    s, z = _lib.as_f32(state), _lib.as_f32(size[..., :2])
-    box = torch.empty(s.shape[:-1] + (5,), dtype=torch.float32, device=s.device)
-    _lib.check(lib.tds_agent_boxes(_lib.ptr(s), _lib.ptr(z), s[..., 0].numel(), _lib.ptr(box), None, None, _lib.stream_ptr(s.device)))
-    return box
+    return ops._agent_boxes(state, size)
 
 
 @agent_boxes.register_fake
@@ -187,12 +139,5 @@ def _(state, size):
     return state.new_empty(state.shape[:-1] + (5,), dtype=torch.float32)
 
 
-def _box_backward(ctx, g):
-    gs = torch.cat([g[..., 0:2], g[..., 4:5], torch.zeros_like(g[..., 0:1])], dim=-1)
-    gz = g[..., 2:4]
-    if ctx.size_cols > 2:
-        gz = torch.cat([gz, g.new_zeros(gz.shape[:-1] + (ctx.size_cols - 2,))], dim=-1)
-    return gs, gz
-
-
-agent_boxes.register_autograd(_box_backward, setup_context=lambda ctx, inputs, output: setattr(ctx, "size_cols", inputs[1].shape[-1]))
+agent_boxes.register_autograd(lambda ctx, g: ops._agent_boxes_grad(g, ctx.size_cols),
+                              setup_context=lambda ctx, inputs, output: setattr(ctx, "size_cols", inputs[1].shape[-1]))
