@@ -299,6 +299,32 @@ int tds_nearest_map_segments_bwd(const tds_map_t* const* maps, int32_t n_maps, c
                                  int32_t k, float* d_grad_state, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Range scan (no counterpart in the reference): the distance along R rays of every origin agent to the first agent box
+ * edge or lane-marking segment.  d_absolute [B,N,6] (x, y, psi, length, width, present) as for tds_agents_relative; the
+ * first A agents are the origins, whatever their present flag.  1 <= R <= 256, max_range finite and > 0.  maps /
+ * n_maps / d_env_map as for tds_nearest_map_segments; n_maps = 0 (maps NULL): agents only.
+ * Ray r of origin i: u = (float32 cospi(2r/R), float32 sinpi(2r/R)) (evaluated in double), (s, c) = sincos(psi_i),
+ * d = (c ux - s uy, s ux + c uy), o = (x_i, y_i).  Candidates: edge k of every agent j != i with present_j != 0, from
+ * corner k to corner (k + 1) % 4 in the corner order of box2corners_th (the corners of tds_offroad_fwd), code 4 j + k;
+ * marking segment s of the map (tds_map_segments), code 4 N + s.  In float32, every operation rounded on its own:
+ *   e = p1 - p0, w = p0 - o, den = dx*ey - dy*ex; den == 0: no hit; t = (wx*ey - wy*ex) / den, u = (wx*dy - wy*dx) / den
+ *   (IEEE division); a hit iff 0 <= u <= 1 and 0 <= t <= max_range (a NaN never hits); a t of -0 counts as +0.
+ * The winner is the smallest (bits(t) << 32 | code).  d_dist [B,A,R] = its t, or max_range without a hit; d_kind
+ * [B,A,R] = 0 for an agent edge, 1 for a marking, -1 for none; d_idx [B,A,R] = j, s or -1.  An origin whose x, y or psi
+ * is not finite hits nothing.  No host synchronisation, no allocation. */
+int tds_range_scan(const tds_map_t* const* maps, int32_t n_maps, const int32_t* d_env_map, const float* d_absolute,
+                   int32_t B, int32_t A, int32_t N, int32_t R, float max_range, float* d_dist, int64_t* d_kind,
+                   int64_t* d_idx, void* stream);
+/* The gradient of d_dist with respect to d_absolute (the map is constant, the selection piecewise constant): d_kind and
+ * d_idx as the forward wrote them, d_grad_dist [B,A,R], d_grad_absolute [B,N,6] (every element is written; the present
+ * column gets 0).  A ray reaches its origin's x, y, psi and, for an agent hit, the hit agent's x, y, psi, length and
+ * width through the winning edge, which is recomputed.  A ray whose kind / idx is not a hit of its row is skipped, not
+ * multiplied by 0.  No atomics: two calls give bit-identical gradients. */
+int tds_range_scan_bwd(const tds_map_t* const* maps, int32_t n_maps, const int32_t* d_env_map, const float* d_absolute,
+                       const int64_t* d_kind, const int64_t* d_idx, const float* d_grad_dist, int32_t B, int32_t A,
+                       int32_t N, int32_t R, float* d_grad_absolute, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Offroad.  Replaces offroad_infraction_loss (infractions.py:176-229) + point_to_mesh_distance_pt
  * (infractions.py:86-173): out[b,a] = sum over the 4 box corners of (d2 if d2 > threshold else 0),
  * d2 = min over ALL map faces of the reference's squared point-triangle distance; times present.

@@ -94,6 +94,10 @@ SIGNATURES = {
                                            c_void_p, c_void_p, c_void_p, c_void_p]),
     "tds_nearest_map_segments_bwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
                                                c_int32, c_int32, c_void_p, c_void_p]),
+    "tds_range_scan": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_float,
+                                 c_void_p, c_void_p, c_void_p, c_void_p]),
+    "tds_range_scan_bwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
+                                     c_int32, c_int32, c_int32, c_void_p, c_void_p]),
     "tds_offroad_fwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                   c_float, c_void_p, c_void_p, c_void_p]),
     "tds_offroad_bwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,

@@ -191,13 +191,8 @@ __device__ float nearest_face(const MapDev& m, float px, float py, float stop, i
 }
 
 __device__ __forceinline__ void corner_of(const float* st, const float* lw, int k, float& px, float& py, float& s, float& c) {
-    // box2corners_th, _iou_utils.py:270-299: (+,+), (-,+), (-,-), (+,-) rotated by psi
-    const float sx = (k == 0 || k == 3) ? 0.5f : -0.5f;
-    const float sy = (k < 2) ? 0.5f : -0.5f;
     tds::sincos_cr(st[2], s, c);
-    const float ux = sx * lw[0], uy = sy * lw[1];
-    px = (ux * c + uy * (-s)) + st[0];
-    py = (ux * s + uy * c) + st[1];
+    tds::box_corner(st[0], st[1], lw[0], lw[1], s, c, k, px, py);
 }
 
 // ---- distance bound of the map (MapDev::obound), built once by tds_map_create.

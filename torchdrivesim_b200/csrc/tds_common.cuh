@@ -44,6 +44,17 @@ __device__ __forceinline__ void sincos_cr(float a, float& s, float& c) {
     c = (float)dc;
 }
 
+// Corner k of the box (x, y, length l, width w) with heading sincos (s, c), in the corner order of box2corners_th
+// (_iou_utils.py:270-299): (+,+), (-,+), (-,-), (+,-) half-extents rotated by psi.  The offroad and range-scan kernels
+// share this arithmetic, so their corners agree bit for bit.
+__device__ __forceinline__ void box_corner(float x, float y, float l, float w, float s, float c, int k, float& px, float& py) {
+    const float sx = (k == 0 || k == 3) ? 0.5f : -0.5f;
+    const float sy = (k < 2) ? 0.5f : -0.5f;
+    const float ux = sx * l, uy = sy * w;
+    px = (ux * c + uy * (-s)) + x;
+    py = (ux * s + uy * c) + y;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

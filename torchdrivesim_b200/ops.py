@@ -4,8 +4,8 @@ Every function takes CUDA tensors in the reference's layouts and launches on the
 stream.  Nothing here has a CPU implementation; `_lib.ptr` raises on CPU tensors.
 
 The differentiable kernels (kinematic step, pairwise and all-pairs collision, agent boxes, relative and nearest-agent
-observations, nearest map segments, offroad) are launched by one private launcher per entry point (`_kinematic_fwd` ...
-`_offroad_bwd`).  The autograd Functions and `out=` paths here,
+observations, nearest map segments, range scan, offroad) are launched by one private launcher per entry point
+(`_kinematic_fwd` ... `_offroad_bwd`).  The autograd Functions and `out=` paths here,
 the custom operators of torch_ops.py and `FusedRollout` all call them.  A launcher checks that the shapes of its inputs
 agree before it touches the library, converts them with the `_lib.as_*` helpers (an input already in the kernel's dtype
 and contiguous is passed through without a copy, which CUDA-graph capture relies on), allocates the outputs it is not
@@ -607,6 +607,110 @@ def nearest_map_segments(state: torch.Tensor, mapset: MapSet, k: int,
     Differentiable in the agent's (x, y, psi) through the filled slots (the map is constant and the selection piecewise
     constant; v gets 0).  One launch each way, no host synchronisation: both directions can be captured in a CUDA graph."""
     return _NearestMapSegments.apply(state, mapset, k, max_distance)
+
+
+def _range_scan_shape(absolute, n_rays, n_agents, mapset):
+    """-> (B, A, N, R): the outputs are [B,A,R]."""
+    if absolute.dim() != 3 or absolute.shape[-1] != 6:
+        raise _lib.TdsError("range_scan: absolute must be [B,N,6]")
+    B, A, N, _ = _agents_relative_shape(absolute, n_agents, False, "range_scan")
+    try:
+        R = operator.index(n_rays)
+    except TypeError:
+        R = 0
+    if not 1 <= R <= 256:
+        raise _lib.TdsError("range_scan: n_rays must be an integer in [1, 256]")
+    if mapset is not None and mapset.env_map is not None and tuple(mapset.env_map.shape) != (B,):
+        raise _lib.TdsError("range_scan: the map set's env_map must be [B]")
+    return B, A, N, R
+
+
+def _range_scan_maps(mapset, device):
+    """(handles, n_maps, env_map) of the map set, (None, 0, None) without one."""
+    if mapset is None:
+        return None, 0, None
+    handles, n_maps = mapset.handles(device)
+    return handles, n_maps, mapset.env_map_on(device)
+
+
+def _range_scan_fwd(absolute, n_rays, n_agents, max_range, mapset):
+    """-> (dist [B,A,R] float32, kind [B,A,R] int64, idx [B,A,R] int64)."""
+    B, A, N, R = _range_scan_shape(absolute, n_rays, n_agents, mapset)
+    try:
+        r = ctypes.c_float(float(max_range)).value
+    except TypeError:
+        r = math.nan
+    if not (math.isfinite(r) and r > 0):
+        raise _lib.TdsError("range_scan: max_range must be finite and > 0 in float32")
+    a = _lib.as_f32(absolute)
+    dist = torch.empty(B, A, R, dtype=torch.float32, device=a.device)
+    kind = torch.empty(B, A, R, dtype=torch.int64, device=a.device)
+    idx = torch.empty(B, A, R, dtype=torch.int64, device=a.device)
+    handles, n_maps, env_map = _range_scan_maps(mapset, a.device)
+    _lib.check(_lib.load().tds_range_scan(handles, n_maps, _lib.ptr(env_map), _lib.ptr(a), B, A, N, R, r, _lib.ptr(dist),
+                                          _lib.ptr(kind), _lib.ptr(idx), _lib.stream_ptr(a.device)))
+    return dist, kind, idx
+
+
+def _range_scan_bwd(absolute, n_rays, n_agents, mapset, kind, idx, grad):
+    """-> d absolute [B,N,6] float32 (the present column gets 0); every element is written by the kernel."""
+    B, A, N, R = _range_scan_shape(absolute, n_rays, n_agents, mapset)
+    for name, t in (("kind", kind), ("idx", idx)):
+        if tuple(t.shape) != (B, A, R) or t.dtype != torch.int64:
+            raise _lib.TdsError(f"range_scan: {name} must be int64 [B,A,R] = {[B, A, R]}")
+    if tuple(grad.shape) != (B, A, R):
+        raise _lib.TdsError(f"range_scan: the gradient must be [B,A,R] = {[B, A, R]}")
+    a, g = _lib.as_f32(absolute), _lib.as_f32(grad)
+    k, i = kind.detach().contiguous(), idx.detach().contiguous()
+    ga = torch.empty_like(a)
+    handles, n_maps, env_map = _range_scan_maps(mapset, a.device)
+    _lib.check(_lib.load().tds_range_scan_bwd(handles, n_maps, _lib.ptr(env_map), _lib.ptr(a), _lib.ptr(k), _lib.ptr(i),
+                                              _lib.ptr(g), B, A, N, R, _lib.ptr(ga), _lib.stream_ptr(a.device)))
+    return ga
+
+
+class _RangeScan(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, absolute, n_rays, n_agents, max_range, mapset):
+        dist, kind, idx = _range_scan_fwd(absolute, n_rays, n_agents, max_range, mapset)
+        ctx.save_for_backward(absolute, kind, idx)
+        ctx.meta = (n_rays, n_agents, mapset)
+        ctx.mark_non_differentiable(kind, idx)
+        return dist, kind, idx
+
+    @staticmethod
+    def backward(ctx, grad_dist, grad_kind, grad_idx):
+        absolute, kind, idx = ctx.saved_tensors
+        n_rays, n_agents, mapset = ctx.meta
+        return _range_scan_bwd(absolute, n_rays, n_agents, mapset, kind, idx, grad_dist), None, None, None, None
+
+
+def range_scan(absolute: torch.Tensor, n_rays: int, n_agents: Optional[int] = None, max_range: float = 50.0,
+               mapset: Optional[MapSet] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The distance along `n_rays` rays of every origin agent to the first agent box or lane marking:
+    absolute [B,N,6] (x, y, psi, length, width, present; get_all_agents_absolute) -> (dist [B,A,R] float32,
+    kind [B,A,R] int64, idx [B,A,R] int64).  The origins are the first A = `n_agents` rows (default N), each computed
+    whatever its own present flag; 1 <= R = n_rays <= 256; `max_range` is finite and > 0 and used as float32(max_range).
+    With `mapset` (`mapset.maps[env_map[b]]` the map of environment b) the lane markings are candidates too.
+
+    Ray r of origin i has the unit vector u_r = (cos, sin)(2 pi r / R) in the agent's frame (the frame of
+    `agents_relative`), evaluated in double with sincospi(2r/R) and rounded to float32, so rays at quarter turns are
+    exact axis vectors.  With (s, c) = sincos(psi_i) (double, rounded), the world direction is d = (c ux - s uy,
+    s ux + c uy) and the origin o = (x_i, y_i).  The candidates are segments: edge k of the box of every agent j != i of
+    the environment with present_j != 0, from corner k to corner (k + 1) % 4 (the corners of `offroad`, in the order of
+    box2corners_th), code 4 j + k; with a map, every lane-marking segment s of `StaticMap.marking_segments`, code
+    4 N + s.  The hit test is float32 with every operation rounded on its own and IEEE division: e = p1 - p0, w = p0 - o,
+    den = dx ey - dy ex; den == 0 is no hit; else t = (wx ey - wy ex) / den, u = (wx dy - wy dx) / den, and it is a hit
+    iff 0 <= u <= 1 and 0 <= t <= float32(max_range).  A NaN never hits; a t of -0 counts as +0.  The winner is the
+    smallest word (bits(t) << 32) | code: the nearest hit, on equal t the smaller code.  dist is its t, or
+    float32(max_range) without a hit; kind is 0 for an agent edge, 1 for a marking, -1 for none; idx is the agent row j,
+    the segment index s, or -1.  An origin whose x, y or psi is not finite hits nothing.
+
+    dist is differentiable in `absolute`: the origin's x, y, psi and, for an agent hit, the hit agent's x, y, psi, length
+    and width (the map is constant, the present column gets 0, the selection is piecewise constant).  A ray without a
+    hit contributes nothing, not even a NaN upstream value.  One launch each way, no host synchronisation: both
+    directions can be captured in a CUDA graph.  Output per origin: 20 bytes per ray."""
+    return _RangeScan.apply(absolute, n_rays, n_agents, max_range, mapset)
 
 
 # ------------------------------------------------------------------------------------ raster

@@ -397,6 +397,15 @@ class Simulator:
         (x, y, psi), and through the kinematic step the actions."""
         return ops.nearest_map_segments(self.get_state(), self.road_mesh, k, max_distance)
 
+    def get_range_scan(self, n_rays: int, max_range: float = 50.0, markings: bool = True) -> Tuple[Tensor, Tensor, Tensor]:
+        """(BxAxR, BxAxR int64, BxAxR int64): the distance along `n_rays` evenly spaced rays of every controlled agent (in
+        its frame, ray 0 straight ahead) to the first box of another present agent or NPC, or with `markings` the first
+        lane-marking segment of the road mesh, up to `max_range`; the kind of the hit (0 agent, 1 marking, -1 none) and
+        its index into get_all_agents_absolute or `StaticMap.marking_segments` (see ops.range_scan).  Differentiable: the
+        gradient reaches the states and sizes, and through the kinematic step the actions."""
+        return ops.range_scan(self.get_all_agents_absolute(), n_rays, self.agent_count, max_range,
+                              self.road_mesh if markings else None)
+
     # ---- noisy observations (simulator.py:663-679, 740-746, 784-821): what every agent perceives of all agents
     def get_noisy_state(self) -> Tensor:
         return self.observation_noise_model.get_noisy_state(self)
