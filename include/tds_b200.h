@@ -325,6 +325,41 @@ int tds_range_scan_bwd(const tds_map_t* const* maps, int32_t n_maps, const int32
                        int32_t N, int32_t R, float* d_grad_absolute, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Time to collision (TTC; no counterpart in the reference): the first contact of every origin agent with any other
+ * present agent under constant velocity, all pairs.
+ * Inputs: d_state [B,N,4] (x, y, psi, v), d_size [B,N,2] (length, width), d_present [B,N] uint8 (0 / non-0);
+ * n_agents = A <= N: rows 0..A-1 are the origins, all N rows are candidates (NPCs take part, as in compute_collision);
+ * horizon H in seconds, finite and > 0.
+ * Every agent keeps its heading and its speed: box j at time t has centre (x_j + t vx_j, y_j + t vy_j), with
+ * vx_j = v_j c_j, vy_j = v_j s_j and (s_j, c_j) = sincos_cr(psi_j) (double precision, rounded), the heading evaluation
+ * the whole path uses.  This is a definition, not the kinematic model's prediction: the bicycle's slip angle is ignored.
+ * Pair (i, j), j != i with both present, float32, every operation rounded on its own (-fmad=false), IEEE division.
+ * The four separating axes, in this order: 1. u_i = (c_i, s_i), 2. u_i⊥ = (-s_i, c_i), 3. u_j, 4. u_j⊥.
+ * For axis n = (nx, ny): d0 = nx (x_j - x_i) + ny (y_j - y_i), s = nx (vx_j - vx_i) + ny (vy_j - vy_i), R = h_i + h_j.
+ * A box's half-extent on its own axes is exactly 0.5 length or 0.5 width; on the other box's axes it is
+ * |n·u| 0.5 length + |n·u⊥| 0.5 width (n·u = nx ux + ny uy).
+ * Entry and exit per axis: s != 0: ta = (-R - d0) / s, tb = (R - d0) / s, entry min(ta, tb), exit max(ta, tb);
+ * s == 0: entry -inf and exit +inf when |d0| <= R, otherwise the pair never touches.
+ * T_in = max of the four entries, T_out = min of the four exits.  The pair touches within the horizon iff
+ * max(T_in, 0) <= min(T_out, H); its time is T_in > 0 ? T_in : +0.0f (no negative zero: keys order by their bits).
+ * Boxes that overlap at t = 0 give 0.  A pair whose time is NaN (a NaN entry or exit) never counts.
+ * Outputs: d_ttc [B,A] float32 and d_idx [B,A] int64, the minimum over j of the pair time, ties to the smaller j (the
+ * key is bits(t) << 32 | j).  No pair touches, or origin i is absent: ttc = +inf, idx = -1.
+ * No host synchronisation, no allocation. */
+int tds_time_to_collision(const float* d_state, const float* d_size, const uint8_t* d_present, int32_t B, int32_t A,
+                          int32_t N, float horizon, float* d_ttc, int64_t* d_idx, void* stream);
+/* The gradient of ttc with respect to the (x, y, psi, v) and (length, width) of the origin and of agent idx, where
+ * 0 < ttc < inf.  There ttc = -(d0 + sgn(s) R) / s on the first axis, in the order above, whose entry equals T_in:
+ * dt/dd0 = -1/s, dt/dR = -1/|s|, dt/ds = -t/s, chained through d0, s and R to both agents (d|x|/dx = sgn(x), 0 at 0).
+ * d_idx as the forward wrote it; the pair and its axis are recomputed from the inputs.  d_grad_ttc [B,A],
+ * d_grad_state [B,N,4], d_grad_size [B,N,2]: every element is written.  A row whose recomputed time is 0 or whose idx
+ * is -1 (or not another present agent) is skipped by a branch, so an inf or NaN upstream value there reaches no
+ * gradient.  No atomics: two calls give bit-identical gradients. */
+int tds_time_to_collision_bwd(const float* d_state, const float* d_size, const uint8_t* d_present, int32_t B,
+                              int32_t A, int32_t N, float horizon, const float* d_grad_ttc, const int64_t* d_idx,
+                              float* d_grad_state, float* d_grad_size, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Offroad.  Replaces offroad_infraction_loss (infractions.py:176-229) + point_to_mesh_distance_pt
  * (infractions.py:86-173): out[b,a] = sum over the 4 box corners of (d2 if d2 > threshold else 0),
  * d2 = min over ALL map faces of the reference's squared point-triangle distance; times present.

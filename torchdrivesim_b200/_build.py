@@ -11,7 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 OUT_DIR = os.path.join(_HERE, "_build")
 LIB_PATH = os.path.join(OUT_DIR, "libtds_b200.so")
-SOURCES = ["common.cu", "kinematic.cu", "collision.cu", "map.cu", "map_segments.cu", "offroad.cu", "range_scan.cu", "raster.cu", "raster_g32.cu", "raster_g128.cu", "raster_g256.cu", "rollout.cu"]
+SOURCES = ["common.cu", "kinematic.cu", "collision.cu", "map.cu", "map_segments.cu", "offroad.cu", "range_scan.cu", "raster.cu", "raster_g32.cu", "raster_g128.cu", "raster_g256.cu", "rollout.cu", "time_to_collision.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     # every fp32 mul/add separately rounded, as the reference's eager CPU ops (see csrc/tds_common.cuh)

@@ -98,6 +98,10 @@ SIGNATURES = {
                                  c_void_p, c_void_p, c_void_p, c_void_p]),
     "tds_range_scan_bwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
                                      c_int32, c_int32, c_int32, c_void_p, c_void_p]),
+    "tds_time_to_collision": (c_int32, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_float, c_void_p,
+                                        c_void_p, c_void_p]),
+    "tds_time_to_collision_bwd": (c_int32, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_float, c_void_p,
+                                            c_void_p, c_void_p, c_void_p, c_void_p]),
     "tds_offroad_fwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                   c_float, c_void_p, c_void_p, c_void_p]),
     "tds_offroad_bwd": (c_int32, [POINTER(c_void_p), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,

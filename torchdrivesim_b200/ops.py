@@ -4,8 +4,8 @@ Every function takes CUDA tensors in the reference's layouts and launches on the
 stream.  Nothing here has a CPU implementation; `_lib.ptr` raises on CPU tensors.
 
 The differentiable kernels (kinematic step, pairwise and all-pairs collision, agent boxes, relative and nearest-agent
-observations, nearest map segments, range scan, offroad) are launched by one private launcher per entry point
-(`_kinematic_fwd` ... `_offroad_bwd`).  The autograd Functions and `out=` paths here,
+observations, nearest map segments, range scan, time to collision, offroad) are launched by one private launcher per
+entry point (`_kinematic_fwd` ... `_offroad_bwd`).  The autograd Functions and `out=` paths here,
 the custom operators of torch_ops.py and `FusedRollout` all call them.  A launcher checks that the shapes of its inputs
 agree before it touches the library, converts them with the `_lib.as_*` helpers (an input already in the kernel's dtype
 and contiguous is passed through without a copy, which CUDA-graph capture relies on), allocates the outputs it is not
@@ -711,6 +711,112 @@ def range_scan(absolute: torch.Tensor, n_rays: int, n_agents: Optional[int] = No
     hit contributes nothing, not even a NaN upstream value.  One launch each way, no host synchronisation: both
     directions can be captured in a CUDA graph.  Output per origin: 20 bytes per ray."""
     return _RangeScan.apply(absolute, n_rays, n_agents, max_range, mapset)
+
+
+# ------------------------------------------------------------------------------------ time to collision
+def _ttc_shape(state, size, present, n_agents, horizon):
+    """-> (B, A, N, H): the outputs are [B,A]; H = float32(horizon), finite and > 0."""
+    if state.dim() != 3 or state.shape[-1] != 4:
+        raise _lib.TdsError("time_to_collision: state must be [B,N,4]")
+    B, N = state.shape[0], state.shape[1]
+    if tuple(size.shape) != (B, N, 2):
+        raise _lib.TdsError(f"time_to_collision: size must be [B,N,2] = {[B, N, 2]}")
+    if tuple(present.shape) != (B, N):
+        raise _lib.TdsError(f"time_to_collision: present must be [B,N] = {[B, N]}")
+    try:
+        A = N if n_agents is None else operator.index(n_agents)
+    except TypeError:
+        A = -1
+    if not 0 <= A <= N:
+        raise _lib.TdsError("time_to_collision: n_agents must be an integer in [0, N]")
+    try:
+        H = ctypes.c_float(float(horizon)).value
+    except TypeError:
+        H = math.nan
+    if not (math.isfinite(H) and H > 0):
+        raise _lib.TdsError("time_to_collision: horizon must be finite and > 0 in float32")
+    return B, A, N, H
+
+
+def _time_to_collision_fwd(state, size, present, n_agents, horizon):
+    """-> (ttc [B,A] float32, idx [B,A] int64); every element is written by the kernel."""
+    B, A, N, H = _ttc_shape(state, size, present, n_agents, horizon)
+    s, z, p = _lib.as_f32(state), _lib.as_f32(size), _lib.as_u8(present)
+    ttc = torch.empty(B, A, dtype=torch.float32, device=s.device)
+    idx = torch.empty(B, A, dtype=torch.int64, device=s.device)
+    _lib.check(_lib.load().tds_time_to_collision(_lib.ptr(s), _lib.ptr(z), _lib.ptr(p), B, A, N, H, _lib.ptr(ttc),
+                                                 _lib.ptr(idx), _lib.stream_ptr(s.device)))
+    return ttc, idx
+
+
+def _time_to_collision_bwd(state, size, present, n_agents, horizon, idx, grad):
+    """-> (d state [B,N,4], d size [B,N,2]) float32; every element is written by the kernel."""
+    B, A, N, H = _ttc_shape(state, size, present, n_agents, horizon)
+    if tuple(idx.shape) != (B, A) or idx.dtype != torch.int64:
+        raise _lib.TdsError(f"time_to_collision: idx must be int64 [B,A] = {[B, A]}")
+    if tuple(grad.shape) != (B, A):
+        raise _lib.TdsError(f"time_to_collision: the gradient must be [B,A] = {[B, A]}")
+    s, z, p = _lib.as_f32(state), _lib.as_f32(size), _lib.as_u8(present)
+    g, i = _lib.as_f32(grad), idx.detach().contiguous()
+    gs, gz = torch.empty_like(s), torch.empty_like(z)
+    _lib.check(_lib.load().tds_time_to_collision_bwd(_lib.ptr(s), _lib.ptr(z), _lib.ptr(p), B, A, N, H, _lib.ptr(g),
+                                                     _lib.ptr(i), _lib.ptr(gs), _lib.ptr(gz), _lib.stream_ptr(s.device)))
+    return gs, gz
+
+
+class _TimeToCollision(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, state, size, present, horizon, n_agents):
+        ttc, idx = _time_to_collision_fwd(state, size, present, n_agents, horizon)
+        ctx.save_for_backward(state, size, present, idx)
+        ctx.meta = (n_agents, horizon)
+        ctx.mark_non_differentiable(idx)
+        return ttc, idx
+
+    @staticmethod
+    def backward(ctx, grad_ttc, grad_idx):
+        state, size, present, idx = ctx.saved_tensors
+        n_agents, horizon = ctx.meta
+        gs, gz = _time_to_collision_bwd(state, size, present, n_agents, horizon, idx, grad_ttc)
+        return gs, gz, None, None, None
+
+
+def time_to_collision(state: torch.Tensor, size: torch.Tensor, present: torch.Tensor, horizon: float = 5.0,
+                      n_agents: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Time to collision (TTC): the first contact of every origin agent under constant velocity, all pairs ->
+    (ttc [B,A] float32, idx [B,A] int64).
+
+    Inputs: state [B,N,4] (x, y, psi, v); size [B,N,2] (length, width); present [B,N] bool; n_agents = A <= N (default
+    N): rows 0..A-1 are the origins, all N rows are candidates, so NPCs take part, as in compute_collision; horizon H in
+    seconds, finite and > 0, used as float32(horizon).
+
+    Every agent keeps its heading and its speed: box j at time t has centre (x_j + t * vx_j, y_j + t * vy_j), with
+    vx_j = v_j * c_j, vy_j = v_j * s_j, and (s_j, c_j) = sincos_cr(psi_j) (double precision, rounded to float32), which
+    is the heading evaluation the whole path uses.  This is a definition, not the kinematic model's prediction: the
+    bicycle's slip angle is ignored, as every TTC metric does.
+
+    Pair (i, j), for j != i with both present, uses float32 arithmetic.  Every operation is rounded on its own (the
+    library is -fmad=false) and divisions are IEEE.  The four separating axes are taken in this order:
+    1. u_i = (c_i, s_i),  2. u_i⊥ = (-s_i, c_i),  3. u_j,  4. u_j⊥.
+    For axis n = (nx, ny): d0 = nx * (x_j - x_i) + ny * (y_j - y_i), s = nx * (vx_j - vx_i) + ny * (vy_j - vy_i),
+    R = h_i + h_j.  A box's half-extent on its own axes is exactly 0.5 * length or 0.5 * width.  On the other box's
+    axes it is |n·u| * 0.5 * length + |n·u⊥| * 0.5 * width.
+    Entry and exit times per axis: if s != 0, ta = (-R - d0) / s and tb = (R - d0) / s, entry min(ta, tb) and exit
+    max(ta, tb); if s == 0, entry is -inf and exit +inf when |d0| <= R, otherwise the pair never touches.
+    T_in is the maximum of the four entries and T_out the minimum of the four exits.  The pair touches within the
+    horizon iff max(T_in, 0) <= min(T_out, H).  Its time is T_in > 0 ? T_in : +0.0 (no negative zero, so keys order by
+    their bits).  Boxes that overlap at t = 0 give 0.  A pair whose time is NaN never counts.
+
+    ttc and idx are the minimum over j of the pair time, ties going to the smaller j (the key is bits(t) << 32 | j).
+    If no pair touches, or origin i is absent: ttc = +inf and idx = -1.
+
+    ttc is differentiable in the (x, y, psi, v) and (length, width) of the origin and of agent idx, where
+    0 < ttc < inf.  There ttc = -(d0 + sgn(s) R) / s on the first axis, in the order above, whose entry equals T_in,
+    with dt/dd0 = -1/s, dt/dR = -1/|s| and dt/ds = -t/s, chained through d0, s and R to both agents (the derivative of
+    |x| is sgn(x), 0 at 0).  Rows with ttc == 0 or idx == -1 are skipped by a branch, so an inf or NaN upstream value
+    there never reaches a gradient.  One launch each way, no host synchronisation: both directions can be captured in
+    a CUDA graph."""
+    return _TimeToCollision.apply(state, size, present, horizon, n_agents)
 
 
 # ------------------------------------------------------------------------------------ raster

@@ -406,6 +406,14 @@ class Simulator:
         return ops.range_scan(self.get_all_agents_absolute(), n_rays, self.agent_count, max_range,
                               self.road_mesh if markings else None)
 
+    def compute_time_to_collision(self, horizon: float = 5.0) -> Tuple[Tensor, Tensor]:
+        """(BxA, BxA int64): the time to collision of every controlled agent within `horizon` seconds when every agent
+        and NPC keeps its heading and speed, and the index of the agent or NPC it meets first (into
+        get_all_agent_state), or (+inf, -1) (see ops.time_to_collision).  Differentiable: the gradient reaches the
+        states and sizes of both agents of each contact, and through the kinematic step the actions."""
+        return ops.time_to_collision(self.get_all_agent_state(), self.get_all_agent_size()[..., :2],
+                                     self.get_all_agent_present_mask(), horizon, self.agent_count)
+
     # ---- noisy observations (simulator.py:663-679, 740-746, 784-821): what every agent perceives of all agents
     def get_noisy_state(self) -> Tensor:
         return self.observation_noise_model.get_noisy_state(self)

@@ -10,6 +10,7 @@ not a tensor.
     torch.ops.tds_b200.agent_boxes(state, size) -> boxes
     torch.ops.tds_b200.agents_relative(absolute, n_agents, exclude_self) -> relative   (absolute [B,N,6] or [B,A,N,6])
     torch.ops.tds_b200.nearest_agents_relative(absolute, k, n_agents, max_distance) -> (relative [B,A,k,6], idx [B,A,k])
+    torch.ops.tds_b200.time_to_collision(state, size, present, horizon, n_agents) -> (ttc [B,A], idx [B,A])
 
 This module holds the registrations only: every operator body calls the launcher of ops.py that the autograd Functions
 use too, so both check their inputs and launch the kernels the same way.
@@ -207,3 +208,42 @@ def _nearest_backward(ctx, g_out, g_idx):
 
 
 nearest_agents_relative.register_autograd(_nearest_backward, setup_context=_nearest_setup)
+
+
+# ------------------------------------------------------------------------------------ time to collision
+@torch.library.custom_op(f"{_NS}::time_to_collision", mutates_args=())
+def time_to_collision(state: Tensor, size: Tensor, present: Tensor, horizon: float, n_agents: Optional[int]) -> Tuple[Tensor, Tensor]:
+    return ops._time_to_collision_fwd(state, size, present, n_agents, horizon)
+
+
+@time_to_collision.register_fake
+def _(state, size, present, horizon, n_agents):
+    B, A, N, H = ops._ttc_shape(state, size, present, n_agents, horizon)
+    return state.new_empty((B, A), dtype=torch.float32), state.new_empty((B, A), dtype=torch.int64)
+
+
+@torch.library.custom_op(f"{_NS}::time_to_collision_backward", mutates_args=())
+def time_to_collision_backward(grad_out: Tensor, state: Tensor, size: Tensor, present: Tensor, idx: Tensor, horizon: float,
+                               n_agents: Optional[int]) -> Tuple[Tensor, Tensor]:
+    return ops._time_to_collision_bwd(state, size, present, n_agents, horizon, idx, grad_out)
+
+
+@time_to_collision_backward.register_fake
+def _(grad_out, state, size, present, idx, horizon, n_agents):
+    return torch.empty_like(state, dtype=torch.float32), torch.empty_like(size, dtype=torch.float32)
+
+
+def _ttc_setup(ctx, inputs, output):
+    state, size, present, horizon, n_agents = inputs
+    ctx.save_for_backward(state, size, present, output[1])
+    ctx.meta = (horizon, n_agents)
+    ctx.mark_non_differentiable(output[1])
+
+
+def _ttc_backward(ctx, g_ttc, g_idx):
+    state, size, present, idx = ctx.saved_tensors
+    gs, gz = time_to_collision_backward(g_ttc.contiguous(), state, size, present, idx, *ctx.meta)
+    return gs, gz, None, None, None
+
+
+time_to_collision.register_autograd(_ttc_backward, setup_context=_ttc_setup)
