@@ -15,6 +15,7 @@
 #include <cooperative_groups.h>
 #include <math_constants.h>
 
+#include "tds_colsum.cuh"
 #include "tds_common.cuh"
 #include "tds_nearest.cuh"
 
@@ -398,7 +399,6 @@ __global__ void __launch_bounds__(kRelWarps * 32) agents_relative_bwd_per_origin
 // are packed into one 64-bit word, key bits above j, and a non-negative float orders like its bit pattern, so the
 // words are distinct and order like the pairs.  Slots past the eligible candidates are zero with index -1.
 constexpr int kNearWarps = 8;                 // warps per CTA of the nearest-agent kernels
-constexpr int kNearCols = 512;                // columns per pass of the shared-mode backward (24 B per column and warp)
 using tds::kNearEmpty;
 
 // One warp per origin row (b, i).  The warp keeps the k smallest words seen so far as a sorted list in registers
@@ -496,12 +496,11 @@ __global__ void __launch_bounds__(kNearWarps * 32) nearest_agents_relative_bwd_p
     }
 }
 
-// Backward, shared mode (absolute [B,N,6]): one CTA per environment, columns in passes of up to kNearCols.  Each warp
-// has a [cols][6] accumulator in shared memory and takes origin rows i = warp, warp + 8, ...; its lanes take the row's
-// slots and add the observed terms of slot (i, s) to the accumulator of column j (distinct within a row; a __syncwarp
-// separates the rows).  In the pass that holds column i, the row's origin terms are summed by a shuffle tree and added
-// to column i too.  The 8 accumulators are then added in warp order and written.  So a column sums its terms in an
-// order fixed by the code: by warp, within a warp by row.  Memory is O(B A k + B N); no dense [B,A,N,6] is formed.
+// Backward, shared mode (absolute [B,N,6]): one CTA per environment, a tds::ColSums column sum (tds_colsum.cuh).  Each
+// warp takes origin rows i = warp, warp + 8, ...; its lanes take the row's slots and add the observed terms of slot
+// (i, s) to the accumulator of column j directly (distinct within a row; a __syncwarp separates the rows).  In the pass
+// that holds column i, the row's origin terms are summed by a shuffle tree and added to column i too.  Memory is
+// O(B A k + B N); no dense [B,A,N,6] is formed.
 __global__ void __launch_bounds__(kNearWarps * 32) nearest_agents_relative_bwd_kernel(
     const float* __restrict__ absolute, const int64_t* __restrict__ idx, const float* __restrict__ gout, int A, int N,
     int k, int cols, float* __restrict__ gabs) {
@@ -512,11 +511,10 @@ __global__ void __launch_bounds__(kNearWarps * 32) nearest_agents_relative_bwd_k
     const int64_t* ib = idx + b * A * (int64_t)k;
     const float* gb = gout + b * A * (int64_t)k * 6;
     float* gw = gabs + b * N * 6;
-    float* acc = s_acc + warp * cols * 6;
+    const tds::ColSums<kNearWarps, 6> sums(s_acc, cols, warp);
     for (int n0 = 0; n0 < N; n0 += cols) {
         const int nc = min(cols, N - n0);
-        for (int q = lane; q < 6 * nc; q += 32) acc[q] = 0.0f;
-        __syncwarp();
+        sums.zero(nc, lane);
         for (int i = warp; i < A; i += kNearWarps) {
             const bool own = i >= n0 && i < n0 + nc;               // warp-uniform: the origin's column is in this pass
             const float* o = ab + (int64_t)i * 6;
@@ -538,7 +536,7 @@ __global__ void __launch_bounds__(kNearWarps * 32) nearest_agents_relative_bwd_k
                 py += t.ty;
                 pp += t.tpsi;
                 if (col) {
-                    float* a = acc + (j - n0) * 6;
+                    float* a = sums.acc + (j - n0) * 6;
                     a[0] += t.tx;
                     a[1] += t.ty;
                     a[2] += g23.x;
@@ -553,7 +551,7 @@ __global__ void __launch_bounds__(kNearWarps * 32) nearest_agents_relative_bwd_k
                 pp = tds::warp_sum(pp);
                 __syncwarp();
                 if (lane == 0) {
-                    float* a = acc + (i - n0) * 6;
+                    float* a = sums.acc + (i - n0) * 6;
                     a[0] -= px;
                     a[1] -= py;
                     a[2] += pp;
@@ -562,12 +560,8 @@ __global__ void __launch_bounds__(kNearWarps * 32) nearest_agents_relative_bwd_k
             __syncwarp();
         }
         __syncthreads();
-        for (int q = threadIdx.x; q < 6 * nc; q += blockDim.x) {   // coalesced: the pass's columns x 6 values
-            float v = 0.0f;
-#pragma unroll
-            for (int w = 0; w < kNearWarps; w++) v += s_acc[w * cols * 6 + q];
-            gw[(int64_t)n0 * 6 + q] = v;
-        }
+        for (int q = threadIdx.x; q < 6 * nc; q += blockDim.x)     // coalesced: the pass's columns x 6 values
+            gw[(int64_t)n0 * 6 + q] = sums.total(q / 6, q % 6);
         __syncthreads();
     }
 }
@@ -1056,8 +1050,7 @@ extern "C" int tds_sensing_occlusion(const float* d_all_state, const float* d_al
     TDS_REQUIRE(B <= 65535, "sensing_occlusion: B=%d exceeds 65535 (shard the batch)", B);
     const size_t smem = (size_t)N * 3 * sizeof(float);
     TDS_REQUIRE(smem <= 200 * 1024, "sensing_occlusion: N=%d does not fit shared memory", N);
-    if (smem > 48 * 1024)
-        TDS_CUDA_OK(cudaFuncSetAttribute(sensing_occlusion_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int e = tds::allow_dynamic_smem(sensing_occlusion_kernel, smem)) return e;
     sensing_occlusion_kernel<<<dim3(A, B), 128, smem, (cudaStream_t)stream>>>((const float4*)d_all_state, (const float2*)d_all_size,
                                                                              d_base_mask, A, N, d_out);
     TDS_LAUNCH_OK();
@@ -1132,11 +1125,9 @@ extern "C" int tds_nearest_agents_relative_bwd(const float* d_absolute, const in
         nearest_agents_relative_bwd_per_origin_kernel<<<(unsigned)blocks, kNearWarps * 32, 0, (cudaStream_t)stream>>>(
             d_absolute, d_idx, d_grad_out, rows, A, N, k, d_grad_absolute);
     } else {
-        const int cols = std::min(N, kNearCols);
+        const int cols = std::min(N, tds::kColsPerPass);
         const size_t smem = (size_t)kNearWarps * cols * 6 * sizeof(float);
-        if (smem > 48 * 1024)
-            TDS_CUDA_OK(cudaFuncSetAttribute(nearest_agents_relative_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)smem));
+        if (int e = tds::allow_dynamic_smem(nearest_agents_relative_bwd_kernel, smem)) return e;
         nearest_agents_relative_bwd_kernel<<<(unsigned)B, kNearWarps * 32, smem, (cudaStream_t)stream>>>(
             d_absolute, d_idx, d_grad_out, A, N, k, cols, d_grad_absolute);
     }
@@ -1180,19 +1171,9 @@ extern "C" int tds_collision_allpairs_fwd(const float* d_ego_box, const float* d
     const dim3 grid((A + kRowsPerCta - 1) / kRowsPerCta, B);
     const size_t smem = (size_t)N * (metric == TDS_METRIC_DISCS ? 13 : 7) * sizeof(float);
     TDS_REQUIRE(smem <= 200 * 1024, "collision_allpairs: N=%d does not fit shared memory", N);
-    if (metric == TDS_METRIC_DISCS) {
-        if (smem > 48 * 1024)
-            TDS_CUDA_OK(cudaFuncSetAttribute(allpairs_fwd_kernel<TDS_METRIC_DISCS>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        allpairs_fwd_kernel<TDS_METRIC_DISCS><<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(
-            d_ego_box, d_all_box, d_mask, A, N, ego_is_prefix, d_out, d_argmax);
-    } else {
-        if (smem > 48 * 1024)
-            TDS_CUDA_OK(cudaFuncSetAttribute(allpairs_fwd_kernel<TDS_METRIC_IOU>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        allpairs_fwd_kernel<TDS_METRIC_IOU><<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(
-            d_ego_box, d_all_box, d_mask, A, N, ego_is_prefix, d_out, d_argmax);
-    }
+    const auto kernel = metric == TDS_METRIC_DISCS ? allpairs_fwd_kernel<TDS_METRIC_DISCS> : allpairs_fwd_kernel<TDS_METRIC_IOU>;
+    if (int e = tds::allow_dynamic_smem(kernel, smem)) return e;
+    kernel<<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(d_ego_box, d_all_box, d_mask, A, N, ego_is_prefix, d_out, d_argmax);
     TDS_LAUNCH_OK();
     return TDS_OK;
 }
@@ -1210,17 +1191,10 @@ extern "C" int tds_collision_allpairs_bwd(const float* d_ego_box, const float* d
     const dim3 grid((A + kRowsPerCta - 1) / kRowsPerCta, B);
     const size_t smem = (size_t)N * 5 * sizeof(float);
     TDS_REQUIRE(smem <= 200 * 1024, "collision_allpairs_bwd: N=%d does not fit shared memory", N);
-    if (metric == TDS_METRIC_DISCS) {
-        if (smem > 48 * 1024)
-            TDS_CUDA_OK(cudaFuncSetAttribute(allpairs_bwd_kernel<TDS_METRIC_DISCS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        allpairs_bwd_kernel<TDS_METRIC_DISCS><<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(
-            d_ego_box, d_all_box, d_mask, A, N, ego_is_prefix, d_grad_out, d_argmax, d_grad_ego, d_grad_all);
-    } else {
-        if (smem > 48 * 1024)
-            TDS_CUDA_OK(cudaFuncSetAttribute(allpairs_bwd_kernel<TDS_METRIC_IOU>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        allpairs_bwd_kernel<TDS_METRIC_IOU><<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(
-            d_ego_box, d_all_box, d_mask, A, N, ego_is_prefix, d_grad_out, d_argmax, d_grad_ego, d_grad_all);
-    }
+    const auto kernel = metric == TDS_METRIC_DISCS ? allpairs_bwd_kernel<TDS_METRIC_DISCS> : allpairs_bwd_kernel<TDS_METRIC_IOU>;
+    if (int e = tds::allow_dynamic_smem(kernel, smem)) return e;
+    kernel<<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(d_ego_box, d_all_box, d_mask, A, N, ego_is_prefix,
+                                                              d_grad_out, d_argmax, d_grad_ego, d_grad_all);
     TDS_LAUNCH_OK();
     return TDS_OK;
 }

@@ -1,8 +1,6 @@
 // Map observations: the k nearest lane-marking segments of every agent, in the agent's frame (tds_nearest_map_segments)
 // and the gradient of that observation with respect to the agent's pose (tds_nearest_map_segments_bwd).  The segments
 // and their grid are built once per map by tds_map_create (map.cu, tds::SegDev).
-#include <math_constants.h>
-
 #include <cstdint>
 
 #include "tds_map.cuh"
@@ -30,14 +28,10 @@ __device__ __forceinline__ float seg_key(float x, float y, float4 q) {
     return qx * qx + qy * qy;
 }
 
-// One warp per agent (b, a).  The cells are searched ring by ring around the agent's cell (clamped into the grid, so an
-// agent off the map starts at the nearest border cell): ring r is the 8 r cells at Chebyshev distance r.  The lanes take
-// 32 cells of a ring at a time, and a scan of their entry counts deals the cells' entries to the lanes, 32 candidates at
-// a time, whatever the cells hold.  Eligible candidates are words (key bits << 32 | s), kept by tds::near_insert.
-// After ring r every unsearched cell lies outside the searched square, at distance >= dmin from the agent, and every
-// point of a segment in it at distance >= dmin - slack.  The search stops when that bound, lowered by more than the
-// rounding of the float32 keys, exceeds the k-th key (a later segment cannot enter the list, nor tie with its key) or
-// the distance limit, or when no cell is left.
+// One warp per agent (b, a), searching the segment grid around the agent by tds::seg_grid_walk.  Eligible candidates
+// are words (key bits << 32 | s), kept by tds::near_insert.  The search stops when the bound dmin - slack on the
+// unsearched segments, lowered by more than the rounding of the float32 keys, exceeds the k-th key (a later segment
+// cannot enter the list, nor tie with its key) or the distance limit, or when no cell is left.
 template <int R>
 __global__ void __launch_bounds__(kSegWarps * 32) nearest_map_segments_kernel(SegSetDev maps, const int32_t* __restrict__ env_map,
                                                                               const float* __restrict__ state, int64_t rows,
@@ -55,60 +49,21 @@ __global__ void __launch_bounds__(kSegWarps * 32) nearest_map_segments_kernel(Se
     const int last_r = (k - 1) >> 5, last_lane = (k - 1) & 31;
     unsigned long long thr = kNearEmpty;                           // the word in slot k - 1
     if (isfinite(x) && isfinite(y) && m.n > 0) {
-        const int cx = (int)fminf(fmaxf(floorf((x - m.x0) * m.inv), 0.0f), (float)(m.gx - 1));
-        const int cy = (int)fminf(fmaxf(floorf((y - m.y0) * m.inv), 0.0f), (float)(m.gy - 1));
-        const int rmax = max(max(cx, m.gx - 1 - cx), max(cy, m.gy - 1 - cy));
-        for (int r = 0; r <= rmax; r++) {
-            const int ncells = r == 0 ? 1 : 8 * r;
-            for (int c0 = 0; c0 < ncells; c0 += 32) {
-                int beg = 0, cnt = 0;
-                const int q = c0 + lane;
-                if (q < ncells) {
-                    int px = cx, py = cy;
-                    if (r > 0) {
-                        const int side = q / (2 * r), off = q - side * 2 * r;
-                        px = side == 0 ? cx - r + off : side == 1 ? cx + r : side == 2 ? cx + r - off : cx - r;
-                        py = side == 0 ? cy - r : side == 1 ? cy - r + off : side == 2 ? cy + r : cy + r - off;
-                    }
-                    if (px >= 0 && px < m.gx && py >= 0 && py < m.gy) {
-                        const int cell = py * m.gx + px;
-                        beg = m.cell[cell];
-                        cnt = m.cell[cell + 1] - beg;
-                    }
+        tds::seg_grid_walk(
+            m, x, y, lane,
+            [&](int j) {
+                unsigned long long cand = kNearEmpty;
+                if (j >= 0) {
+                    const float key = seg_key(x, y, m.seg[j]);
+                    if (key <= r2) cand = ((unsigned long long)__float_as_uint(key) << 32) | (unsigned)j;
                 }
-                int incl = cnt;                                    // inclusive scan of the lanes' counts
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int v = __shfl_up_sync(0xffffffffu, incl, o);
-                    if (lane >= o) incl += v;
-                }
-                const int total = __shfl_sync(0xffffffffu, incl, 31);
-                for (int t0 = 0; t0 < total; t0 += 32) {
-                    const int t = t0 + lane;
-                    int pos = 0;                                   // the lane whose cell holds entry t: first incl > t
-#pragma unroll
-                    for (int step = 16; step > 0; step >>= 1)
-                        if (__shfl_sync(0xffffffffu, incl, pos + step - 1) <= t) pos += step;
-                    const int cbeg = __shfl_sync(0xffffffffu, beg, pos), cfirst = __shfl_sync(0xffffffffu, incl - cnt, pos);
-                    unsigned long long cand = kNearEmpty;
-                    if (t < total) {
-                        const int j = m.ent[cbeg + t - cfirst];
-                        const float key = seg_key(x, y, m.seg[j]);
-                        if (key <= r2) cand = ((unsigned long long)__float_as_uint(key) << 32) | (unsigned)j;
-                    }
-                    tds::near_insert<R>(list, cand, thr, last_r, last_lane, lane);
-                }
-            }
-            // distance to the unsearched cells (double: exact for float inputs, whatever the map's coordinates)
-            double dmin = CUDART_INF;
-            if (cx - r > 0) dmin = fmin(dmin, (double)x - ((double)m.x0 + (double)(cx - r) * m.cs));
-            if (cx + r < m.gx - 1) dmin = fmin(dmin, ((double)m.x0 + (double)(cx + r + 1) * m.cs) - (double)x);
-            if (cy - r > 0) dmin = fmin(dmin, (double)y - ((double)m.y0 + (double)(cy - r) * m.cs));
-            if (cy + r < m.gy - 1) dmin = fmin(dmin, ((double)m.y0 + (double)(cy + r + 1) * m.cs) - (double)y);
-            // a float32 key errs by far less than 1e-5 of the distance plus 1e-3 m
-            const double lb = (dmin - m.slack) * (1.0 - 1e-5) - 1e-3;
-            if (lb > 0.0 && ((double)__uint_as_float((unsigned)(thr >> 32)) < lb * lb || lb * lb > (double)r2)) break;
-        }
+                tds::near_insert<R>(list, cand, thr, last_r, last_lane, lane);
+            },
+            [&](double dmin) {
+                // a float32 key errs by far less than 1e-5 of the distance plus 1e-3 m
+                const double lb = (dmin - m.slack) * (1.0 - 1e-5) - 1e-3;
+                return lb > 0.0 && ((double)__uint_as_float((unsigned)(thr >> 32)) < lb * lb || lb * lb > (double)r2);
+            });
     }
     // indices and kinds first, the rows after the heading's sincos (an ABI call): the list is not live across it
 #pragma unroll

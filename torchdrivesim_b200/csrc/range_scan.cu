@@ -13,6 +13,7 @@
 #include <cmath>
 #include <cstdint>
 
+#include "tds_colsum.cuh"
 #include "tds_map.cuh"
 #include "tds_nearest.cuh"
 
@@ -24,7 +25,6 @@ using tds::SegSetDev;
 
 constexpr int kScanWarps = 8;            // warps per CTA of the forward (one warp per origin)
 constexpr int kScanCacheAgents = 1024;   // the forward caches an environment's box corners (32 B per agent) up to this N
-constexpr int kScanCols = 512;           // columns per pass of the backward (20 B per column and warp)
 constexpr float kTwoPi = 6.28318530717958647692f;
 
 // (float32 of cospi(2r/R), float32 of sinpi(2r/R)): ray r in the agent's frame, exact axis vectors at quarter turns.
@@ -107,9 +107,9 @@ __device__ __forceinline__ void scan_segment(float ox, float oy, float4 p, unsig
 // warp the world directions d_r and the best word of each ray (64-bit atomicMin: the minimum does not depend on the
 // order of the candidates, so the result is deterministic).  When the CTA's rows belong to one environment and N <=
 // kScanCacheAgents, the environment's box corners are computed once into shared memory (NaN for an absent agent, which
-// then never hits).  The lanes take 32 candidates at a time: first the 4 N box edges, then the markings of the cells
-// of the segment grid ring by ring, dealt as in nearest_map_segments_kernel.  After a ring the search stops when the
-// unsearched cells lie beyond max_range or beyond the t of every ray (by lower_bound), or when no cell is left.
+// then never hits).  The lanes take 32 candidates at a time: first the 4 N box edges, then the markings, walking the
+// segment grid by tds::seg_grid_walk.  After a ring the search stops when the unsearched cells lie beyond max_range or
+// beyond the t of every ray (by lower_bound), or when no cell is left.
 __global__ void __launch_bounds__(kScanWarps * 32) range_scan_kernel(SegSetDev maps, int use_map,
                                                                      const int32_t* __restrict__ env_map,
                                                                      const float* __restrict__ absolute, int64_t rows,
@@ -179,65 +179,26 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_kernel(SegSetDev m
         }
         const SegDev& m = maps.m[env_map ? env_map[b] : 0];
         if (use_map && m.n > 0) {
-            const int cx = (int)fminf(fmaxf(floorf((ox - m.x0) * m.inv), 0.0f), (float)(m.gx - 1));
-            const int cy = (int)fminf(fmaxf(floorf((oy - m.y0) * m.inv), 0.0f), (float)(m.gy - 1));
-            const int rmax = max(max(cx, m.gx - 1 - cx), max(cy, m.gy - 1 - cy));
             const unsigned base = 4u * (unsigned)N;
-            for (int ring = 0; ring <= rmax; ring++) {
-                const int ncells = ring == 0 ? 1 : 8 * ring;
-                for (int c0 = 0; c0 < ncells; c0 += 32) {
-                    int beg = 0, cnt = 0;
-                    const int q = c0 + lane;
-                    if (q < ncells) {
-                        int px = cx, py = cy;
-                        if (ring > 0) {
-                            const int side = q / (2 * ring), off = q - side * 2 * ring;
-                            px = side == 0 ? cx - ring + off : side == 1 ? cx + ring : side == 2 ? cx + ring - off : cx - ring;
-                            py = side == 0 ? cy - ring : side == 1 ? cy - ring + off : side == 2 ? cy + ring : cy + ring - off;
-                        }
-                        if (px >= 0 && px < m.gx && py >= 0 && py < m.gy) {
-                            const int cell = py * m.gx + px;
-                            beg = m.cell[cell];
-                            cnt = m.cell[cell + 1] - beg;
-                        }
-                    }
-                    int incl = cnt;                                // inclusive scan of the lanes' counts
+            tds::seg_grid_walk(
+                m, ox, oy, lane,
+                [&](int sg) {
+                    if (sg >= 0)
+                        scan_segment(ox, oy, m.seg[sg], base + (unsigned)sg, max_range, range_lb2, apsi, R, dirs, best);
+                },
+                [&](double dmin) {
+                    const double lbd = lower_bound(dmin - m.slack);
+                    if (lbd > (double)max_range) return true;
+                    if (lbd > 0.0) {
+                        __syncwarp();
+                        unsigned top = 0;                          // the largest t bits of the rays (no hit: NaN bits)
+                        for (int r = lane; r < R; r += 32) top = max(top, (unsigned)(best[r] >> 32));
 #pragma unroll
-                    for (int o = 1; o < 32; o <<= 1) {
-                        const int v = __shfl_up_sync(0xffffffffu, incl, o);
-                        if (lane >= o) incl += v;
+                        for (int o = 16; o > 0; o >>= 1) top = max(top, __shfl_xor_sync(0xffffffffu, top, o));
+                        if (lbd > (double)__uint_as_float(top)) return true;  // false for NaN
                     }
-                    const int total = __shfl_sync(0xffffffffu, incl, 31);
-                    for (int t0 = 0; t0 < total; t0 += 32) {
-                        const int t = t0 + lane;
-                        int pos = 0;                               // the lane whose cell holds entry t: first incl > t
-#pragma unroll
-                        for (int step = 16; step > 0; step >>= 1)
-                            if (__shfl_sync(0xffffffffu, incl, pos + step - 1) <= t) pos += step;
-                        const int cbeg = __shfl_sync(0xffffffffu, beg, pos), cfirst = __shfl_sync(0xffffffffu, incl - cnt, pos);
-                        if (t < total) {
-                            const int sg = m.ent[cbeg + t - cfirst];
-                            scan_segment(ox, oy, m.seg[sg], base + (unsigned)sg, max_range, range_lb2, apsi, R, dirs, best);
-                        }
-                    }
-                }
-                // distance to the unsearched cells (double: exact for float inputs, whatever the map's coordinates)
-                double dmin = CUDART_INF;
-                if (cx - ring > 0) dmin = fmin(dmin, (double)ox - ((double)m.x0 + (double)(cx - ring) * m.cs));
-                if (cx + ring < m.gx - 1) dmin = fmin(dmin, ((double)m.x0 + (double)(cx + ring + 1) * m.cs) - (double)ox);
-                if (cy - ring > 0) dmin = fmin(dmin, (double)oy - ((double)m.y0 + (double)(cy - ring) * m.cs));
-                if (cy + ring < m.gy - 1) dmin = fmin(dmin, ((double)m.y0 + (double)(cy + ring + 1) * m.cs) - (double)oy);
-                const double lbd = lower_bound(dmin - m.slack);
-                if (lbd > (double)max_range) break;
-                if (lbd > 0.0) {
-                    __syncwarp();
-                    unsigned top = 0;                              // the largest t bits of the rays (no hit: NaN bits)
-                    for (int r = lane; r < R; r += 32) top = max(top, (unsigned)(best[r] >> 32));
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1) top = max(top, __shfl_xor_sync(0xffffffffu, top, o));
-                    if (lbd > (double)__uint_as_float(top)) break;  // false for NaN
-                }
-            }
+                    return false;
+                });
         }
     }
     __syncwarp();
@@ -258,16 +219,16 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_kernel(SegSetDev m
     }
 }
 
-// Backward: one CTA per environment, columns (agents) in passes of up to kScanCols.  Each warp has a [cols][5]
-// accumulator (x, y, psi, length, width) in shared memory and takes origin rows i = warp, warp + 8, ...; its lanes take
-// the row's rays.  A ray's winner is recomputed from kind and idx; with q = g / den:
+// Backward: one CTA per environment, a tds::ColSums column sum (tds_colsum.cuh) over (x, y, psi, length, width).  Each
+// warp takes origin rows i = warp, warp + 8, ...; its lanes take the row's rays.  A ray's winner is recomputed from
+// kind and idx; with q = g / den:
 //   origin:        d x += -ey q,  d y += ex q,  d psi += t (d . e) q;
 //   edge (p0, p1): d p0 += (1 - u) (ey q, -ex q),  d p1 += u (ey q, -ex q),
 // and a corner's gradient (gx, gy) reaches its agent as d x += gx, d y += gy, d psi += -gx ry + gy rx ((rx, ry) the
 // rotated half-extents), d length += sx (gx c + gy s), d width += sy (-gx s + gy c).  The agent terms of the rays are
-// added to the accumulator one lane after the other (several rays may hit one agent); the origin terms are summed per
-// lane over its rays and then by a shuffle tree, and added to column i after the row.  The 8 accumulators are added in
-// warp order.  A ray whose kind / idx is not a hit of this row (no hit, an agent index out of range or i itself, a
+// added to the accumulator by tds::add_lane_serial (several rays may hit one agent); the origin terms are summed per
+// lane over its rays and then by a shuffle tree, and added to column i after the row.  The output's present column
+// gets 0.  A ray whose kind / idx is not a hit of this row (no hit, an agent index out of range or i itself, a
 // marking index out of range) is skipped by a branch, so a NaN upstream value there does not reach the gradient.
 __global__ void __launch_bounds__(kScanWarps * 32) range_scan_bwd_kernel(SegSetDev maps, int use_map,
                                                                          const int32_t* __restrict__ env_map,
@@ -280,7 +241,7 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_bwd_kernel(SegSetD
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t b = blockIdx.x;
     float2* units = reinterpret_cast<float2*>(s_bwd);              // [R]
-    float* acc = s_bwd + 2 * R + warp * cols * 5;                  // [kScanWarps][cols][5]
+    const tds::ColSums<kScanWarps, 5> sums(s_bwd + 2 * R, cols, warp);
     for (int r = threadIdx.x; r < R; r += blockDim.x) units[r] = ray_unit(r, R);
     const float* ab = absolute + b * N * 6;
     float* gw = gabs + b * N * 6;
@@ -289,8 +250,7 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_bwd_kernel(SegSetD
     __syncthreads();
     for (int n0 = 0; n0 < N; n0 += cols) {
         const int nc = min(cols, N - n0);
-        for (int q = lane; q < 5 * nc; q += 32) acc[q] = 0.0f;
-        __syncwarp();
+        sums.zero(nc, lane);
         for (int i = warp; i < A; i += kScanWarps) {
             const bool own = i >= n0 && i < n0 + nc;               // warp-uniform: the origin's column is in this pass
             const float* o = ab + (int64_t)i * 6;
@@ -301,7 +261,7 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_bwd_kernel(SegSetD
             for (int r0 = 0; r0 < R; r0 += 32) {
                 const int r = r0 + lane;
                 const int64_t e = ((int64_t)b * A + i) * R + r;
-                int j = -1;                                        // the hit agent, when its column is in this pass
+                int j[1] = {-1};                                   // the hit agent, when its column is in this pass
                 float v[5] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
                 if (r < R) {
                     const int64_t kd = kind[e], id = idx[e];
@@ -346,7 +306,7 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_bwd_kernel(SegSetD
                             pp += (t * (d.x * ex + d.y * ey)) * q;
                         }
                         if (col) {
-                            j = (int)id;
+                            j[0] = (int)id;
                             const float gx = ey * q, gy = -(ex * q);
                             const float sx0 = (k == 0 || k == 3) ? 0.5f : -0.5f, sy0 = k < 2 ? 0.5f : -0.5f;
                             const int k1 = (k + 1) & 3;
@@ -365,26 +325,14 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_bwd_kernel(SegSetD
                         }
                     }
                 }
-                // the agent terms of the lanes' rays, added lane after lane (several rays may hit one agent)
-                for (unsigned todo = __ballot_sync(0xffffffffu, j >= 0); todo; todo &= todo - 1) {
-                    const int src = __ffs(todo) - 1;
-                    const int jj = __shfl_sync(0xffffffffu, j, src);
-                    float mine = 0.0f;
-#pragma unroll
-                    for (int comp = 0; comp < 5; comp++) {
-                        const float x = __shfl_sync(0xffffffffu, v[comp], src);
-                        if (lane == comp) mine = x;
-                    }
-                    if (lane < 5) acc[(jj - n0) * 5 + lane] += mine;
-                    __syncwarp();
-                }
+                tds::add_lane_serial<5, 1>(sums.acc, n0, j, v, lane);
             }
             if (own) {
                 px = tds::warp_sum(px);
                 py = tds::warp_sum(py);
                 pp = tds::warp_sum(pp);
                 if (lane == 0) {
-                    float* a = acc + (i - n0) * 5;
+                    float* a = sums.acc + (i - n0) * 5;
                     a[0] += px;
                     a[1] += py;
                     a[2] += pp;
@@ -395,12 +343,7 @@ __global__ void __launch_bounds__(kScanWarps * 32) range_scan_bwd_kernel(SegSetD
         __syncthreads();
         for (int q = threadIdx.x; q < 6 * nc; q += blockDim.x) {   // coalesced: the pass's columns x 6 values
             const int n = q / 6, comp = q - n * 6;
-            float v = 0.0f;
-            if (comp < 5) {
-#pragma unroll
-                for (int w = 0; w < kScanWarps; w++) v += s_bwd[2 * R + w * cols * 5 + n * 5 + comp];
-            }
-            gw[(int64_t)n0 * 6 + q] = v;
+            gw[(int64_t)n0 * 6 + q] = comp < 5 ? sums.total(n, comp) : 0.0f;
         }
         __syncthreads();
     }
@@ -425,8 +368,7 @@ extern "C" int tds_range_scan(const tds_map_t* const* maps, int32_t n_maps, cons
     TDS_REQUIRE(blocks <= 2147483647LL, "range_scan: too many agents");
     const size_t smem = (size_t)kScanWarps * R * 8 + (size_t)R * 8 + (size_t)kScanWarps * R * 8 +
                         (N <= kScanCacheAgents ? (size_t)N * 32 : 0);
-    if (smem > 48 * 1024)
-        TDS_CUDA_OK(cudaFuncSetAttribute(range_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int e = tds::allow_dynamic_smem(range_scan_kernel, smem)) return e;
     range_scan_kernel<<<(unsigned)blocks, kScanWarps * 32, smem, (cudaStream_t)stream>>>(
         set, n_maps > 0 ? 1 : 0, n_maps > 0 ? d_env_map : nullptr, d_absolute, rows, A, N, R, max_range, d_dist, d_kind,
         d_idx);
@@ -446,10 +388,9 @@ extern "C" int tds_range_scan_bwd(const tds_map_t* const* maps, int32_t n_maps, 
     }
     if ((int64_t)B * N == 0) return TDS_OK;
     TDS_REQUIRE(d_absolute && d_grad_absolute && (A == 0 || (d_kind && d_idx && d_grad_dist)), "range_scan_bwd: null pointer");
-    const int cols = std::min(N, kScanCols);
+    const int cols = std::min(N, tds::kColsPerPass);
     const size_t smem = (size_t)R * 8 + (size_t)kScanWarps * cols * 5 * sizeof(float);
-    if (smem > 48 * 1024)
-        TDS_CUDA_OK(cudaFuncSetAttribute(range_scan_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int e = tds::allow_dynamic_smem(range_scan_bwd_kernel, smem)) return e;
     range_scan_bwd_kernel<<<(unsigned)B, kScanWarps * 32, smem, (cudaStream_t)stream>>>(
         set, n_maps > 0 ? 1 : 0, n_maps > 0 ? d_env_map : nullptr, d_absolute, d_kind, d_idx, d_grad_dist, A, N, R, cols,
         d_grad_absolute);

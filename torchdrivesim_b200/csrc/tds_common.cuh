@@ -35,6 +35,13 @@ int sm_count();
             return ::tds::fail(TDS_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(_e)); \
     } while (0)
 
+// A launch with more than 48 KB of dynamic shared memory fails unless the kernel opts in first.
+template <class K>
+int allow_dynamic_smem(K kernel, size_t bytes) {
+    if (bytes > 48 * 1024) TDS_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    return TDS_OK;
+}
+
 // sin/cos evaluated in double and rounded to fp32: effectively correctly rounded, hence
 // reproducible on the CPU (the oracle does the same) and within 1 ulp of torch's CPU sin/cos.
 __device__ __forceinline__ void sincos_cr(float a, float& s, float& c) {

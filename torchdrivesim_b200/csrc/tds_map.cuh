@@ -1,5 +1,7 @@
 // Static map acceleration structures (device view).  Built once per map by tds_map_create.
 #pragma once
+#include <math_constants.h>
+
 #include "tds_common.cuh"
 
 namespace tds {
@@ -73,6 +75,72 @@ struct SegDev {
 struct SegSetDev {
     SegDev m[TDS_MAX_MAPS];
 };
+
+// One warp's walk over the segment grid around (x, y), what the map-segment and range-scan kernels search it with.
+// The cells are taken ring by ring around the point's cell (clamped into the grid, so a point off the map starts at the
+// nearest border cell): ring r is the 8 r cells at Chebyshev distance r, in side order.  The lanes take 32 cells of a
+// ring at a time, and a scan of their entry counts deals the cells' entries to the lanes, 32 at a time, whatever the
+// cells hold.  After ring r every unsearched cell lies outside the searched square, at distance >= dmin from (x, y),
+// and every point of a segment listed in it at distance >= dmin - slack.
+// visit(s): called by all 32 lanes once per round of 32 entries; s = segment index, or -1 for a lane with no entry
+//           (so visit may contain warp collectives such as tds::near_insert).
+// done(dmin): called by all 32 lanes after each ring with the double-precision distance from (x, y) to the unsearched
+//           cells (CUDART_INF when none is left on any side); returns a warp-uniform bool: stop.
+// Precondition: x, y finite and m.n > 0.
+template <class Visit, class Done>
+__device__ __forceinline__ void seg_grid_walk(const SegDev& m, float x, float y, int lane, Visit visit, Done done) {
+    const int cx = (int)fminf(fmaxf(floorf((x - m.x0) * m.inv), 0.0f), (float)(m.gx - 1));
+    const int cy = (int)fminf(fmaxf(floorf((y - m.y0) * m.inv), 0.0f), (float)(m.gy - 1));
+    const int rmax = max(max(cx, m.gx - 1 - cx), max(cy, m.gy - 1 - cy));
+    for (int r = 0; r <= rmax; r++) {
+        const int ncells = r == 0 ? 1 : 8 * r;
+        for (int c0 = 0; c0 < ncells; c0 += 32) {
+            int beg = 0, cnt = 0;
+            const int q = c0 + lane;
+            if (q < ncells) {
+                int px = cx, py = cy;
+                if (r > 0) {
+                    const int side = q / (2 * r), off = q - side * 2 * r;
+                    px = side == 0 ? cx - r + off : side == 1 ? cx + r : side == 2 ? cx + r - off : cx - r;
+                    py = side == 0 ? cy - r : side == 1 ? cy - r + off : side == 2 ? cy + r : cy + r - off;
+                }
+                if (px >= 0 && px < m.gx && py >= 0 && py < m.gy) {
+                    const int cell = py * m.gx + px;
+                    beg = m.cell[cell];
+                    cnt = m.cell[cell + 1] - beg;
+                }
+            }
+            int incl = cnt;                                        // inclusive scan of the lanes' counts
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int v = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += v;
+            }
+            const int total = __shfl_sync(0xffffffffu, incl, 31);
+            for (int t0 = 0; t0 < total; t0 += 32) {
+                const int t = t0 + lane;
+                int pos = 0;                                       // the lane whose cell holds entry t: first incl > t
+#pragma unroll
+                for (int step = 16; step > 0; step >>= 1)
+                    if (__shfl_sync(0xffffffffu, incl, pos + step - 1) <= t) pos += step;
+                const int cbeg = __shfl_sync(0xffffffffu, beg, pos), cfirst = __shfl_sync(0xffffffffu, incl - cnt, pos);
+                int s = -1;
+                if (t < total) {
+                    s = m.ent[cbeg + t - cfirst];
+                    __builtin_assume(s >= 0);                      // so that visit's s >= 0 folds into t < total
+                }
+                visit(s);
+            }
+        }
+        // distance to the unsearched cells (double: exact for float inputs, whatever the map's coordinates)
+        double dmin = CUDART_INF;
+        if (cx - r > 0) dmin = fmin(dmin, (double)x - ((double)m.x0 + (double)(cx - r) * m.cs));
+        if (cx + r < m.gx - 1) dmin = fmin(dmin, ((double)m.x0 + (double)(cx + r + 1) * m.cs) - (double)x);
+        if (cy - r > 0) dmin = fmin(dmin, (double)y - ((double)m.y0 + (double)(cy - r) * m.cs));
+        if (cy + r < m.gy - 1) dmin = fmin(dmin, ((double)m.y0 + (double)(cy + r + 1) * m.cs) - (double)y);
+        if (done(dmin)) break;
+    }
+}
 
 }  // namespace tds
 

@@ -16,6 +16,7 @@
 #include <cmath>
 #include <cstdint>
 
+#include "tds_colsum.cuh"
 #include "tds_common.cuh"
 #include "tds_nearest.cuh"
 
@@ -27,7 +28,6 @@ constexpr int kTtcWarps = 8;        // warps per CTA of both kernels
 constexpr int kTtcRows = 64;        // origin rows per CTA of the forward, 8 per warp
 constexpr int kTtcTile = 1024;      // columns staged in shared memory at a time by the forward
 constexpr int kTtcStride = 11;      // floats per staged agent (odd: conflict-free column reads)
-constexpr int kTtcCols = 512;       // columns per pass of the backward (24 B per column and warp)
 
 // What both kernels need of an agent, in the staged order.
 struct TtcAgent {
@@ -244,13 +244,12 @@ __device__ __forceinline__ void ttc_pair_grad(const TtcAgent& I, const TtcAgent&
     goth[5] += 0.5f * (gR * fabsf(a.q));
 }
 
-// Backward: one CTA per environment, columns in passes of up to kTtcCols.  Each warp has a [cols][6] accumulator
-// (x, y, psi, v, length, width) in shared memory and takes origin rows 32 at a time (rows 32 (8 m + warp) + lane).  A
-// lane recomputes its row's contact with agent idx (and so its axis) from the inputs; a row whose contact is not at a
-// time in (0, H] (ttc == 0, idx == -1, an index that is not another present agent) is skipped by a branch, so an inf
-// or NaN upstream value there reaches nothing.  The rows' 12 terms are added to the accumulator one row after the
-// other (origin terms by lanes 0-5, hit-agent terms by lanes 6-11; i != j, so they never meet in one step), and the
-// 8 accumulators are added in warp order.  No atomics: the order of every sum is fixed by the code.
+// Backward: one CTA per environment, a tds::ColSums column sum (tds_colsum.cuh) over (x, y, psi, v, length, width).
+// Each warp takes origin rows 32 at a time (rows 32 (8 m + warp) + lane).  A lane recomputes its row's contact with
+// agent idx (and so its axis) from the inputs; a row whose contact is not at a time in (0, H] (ttc == 0, idx == -1, an
+// index that is not another present agent) is skipped by a branch, so an inf or NaN upstream value there reaches
+// nothing.  The rows' 12 terms are added to the accumulator by tds::add_lane_serial, one row after the other (origin
+// terms by lanes 0-5, hit-agent terms by lanes 6-11; i != j, so they never meet in one step).
 __global__ void __launch_bounds__(kTtcWarps * 32) ttc_bwd_kernel(const float* __restrict__ state,
                                                                  const float* __restrict__ size,
                                                                  const uint8_t* __restrict__ present,
@@ -262,14 +261,13 @@ __global__ void __launch_bounds__(kTtcWarps * 32) ttc_bwd_kernel(const float* __
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t b = blockIdx.x;
     const int64_t base = b * N;
-    float* acc = s_acc + warp * cols * 6;
+    const tds::ColSums<kTtcWarps, 6> sums(s_acc, cols, warp);
     for (int n0 = 0; n0 < N; n0 += cols) {
         const int nc = min(cols, N - n0);
-        for (int q = lane; q < 6 * nc; q += 32) acc[q] = 0.0f;
-        __syncwarp();
+        sums.zero(nc, lane);
         for (int i0 = warp * 32; i0 < A; i0 += kTtcWarps * 32) {
             const int i = i0 + lane;
-            int ci = -1, cj = -1;                                    // the columns this lane's terms go to
+            int cl[2] = {-1, -1};                                    // the columns of the origin and hit-agent terms
             float v[12];
 #pragma unroll
             for (int c = 0; c < 12; c++) v[c] = 0.0f;
@@ -285,31 +283,17 @@ __global__ void __launch_bounds__(kTtcWarps * 32) ttc_bwd_kernel(const float* __
                     const float t = ttc_pair(I, J, H, axis);
                     if (t > 0.0f) {
                         ttc_pair_grad(I, J, axis, t, gout[e], v, v + 6);
-                        ci = own ? i : -1;
-                        cj = col ? (int)j : -1;
+                        cl[0] = own ? i : -1;
+                        cl[1] = col ? (int)j : -1;
                     }
                 }
             }
-            for (unsigned todo = __ballot_sync(0xffffffffu, ci >= 0 || cj >= 0); todo; todo &= todo - 1) {
-                const int src = __ffs(todo) - 1;
-                const int si = __shfl_sync(0xffffffffu, ci, src), sj = __shfl_sync(0xffffffffu, cj, src);
-                float mine = 0.0f;
-#pragma unroll
-                for (int c = 0; c < 12; c++) {
-                    const float x = __shfl_sync(0xffffffffu, v[c], src);
-                    if (lane == c) mine = x;
-                }
-                if (lane < 6 && si >= 0) acc[(si - n0) * 6 + lane] += mine;
-                if (lane >= 6 && lane < 12 && sj >= 0) acc[(sj - n0) * 6 + lane - 6] += mine;
-                __syncwarp();
-            }
+            tds::add_lane_serial<6, 2>(sums.acc, n0, cl, v, lane);
         }
         __syncthreads();
         for (int q = threadIdx.x; q < 6 * nc; q += blockDim.x) {
             const int n = q / 6, comp = q - n * 6;
-            float s = 0.0f;
-#pragma unroll
-            for (int w = 0; w < kTtcWarps; w++) s += s_acc[w * cols * 6 + q];
+            const float s = sums.total(n, comp);
             const int64_t e = base + n0 + n;
             if (comp < 4) gstate[e * 4 + comp] = s;
             else gsize[e * 2 + comp - 4] = s;
@@ -343,10 +327,9 @@ extern "C" int tds_time_to_collision_bwd(const float* d_state, const float* d_si
     if ((int64_t)B * N == 0) return TDS_OK;
     TDS_REQUIRE(d_state && d_size && d_present && d_grad_state && d_grad_size && (A == 0 || (d_grad_ttc && d_idx)),
                 "time_to_collision_bwd: null pointer");
-    const int cols = std::min(N, kTtcCols);
+    const int cols = std::min(N, tds::kColsPerPass);
     const size_t smem = (size_t)kTtcWarps * cols * 6 * sizeof(float);
-    if (smem > 48 * 1024)
-        TDS_CUDA_OK(cudaFuncSetAttribute(ttc_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int e = tds::allow_dynamic_smem(ttc_bwd_kernel, smem)) return e;
     ttc_bwd_kernel<<<(unsigned)B, kTtcWarps * 32, smem, (cudaStream_t)stream>>>(d_state, d_size, d_present, d_grad_ttc,
                                                                                d_idx, A, N, horizon, cols, d_grad_state,
                                                                                d_grad_size);
