@@ -843,7 +843,9 @@ __global__ void __launch_bounds__(256) pairwise_bwd_kernel(const float* __restri
 constexpr int kRowsPerCta = 64;
 constexpr int kWarps = 8;
 
-// shared memory: all N column boxes of the environment, as discs (12 floats) or Box (6 floats)
+// shared memory: all N column boxes of the environment, as discs (12 floats + mask) or Box (6 floats + mask); the
+// discs of the CTA's own rows follow the columns, so that every box goes through make_discs (and its double-precision
+// sincos) once per CTA, all of them at the same time, and the row loop reads nothing but shared memory
 template <int METRIC>
 __global__ void __launch_bounds__(kWarps * 32) allpairs_fwd_kernel(const float* __restrict__ ego, const float* __restrict__ all,
                                                                   const uint8_t* __restrict__ mask, int A, int N,
@@ -856,14 +858,15 @@ __global__ void __launch_bounds__(kWarps * 32) allpairs_fwd_kernel(const float* 
     const int row0 = blockIdx.x * kRowsPerCta;
     const float* allb = all + (size_t)b * N * 5;
     const uint8_t* mb = mask + (size_t)b * N;
-    for (int j = threadIdx.x; j < N; j += blockDim.x) {
-        const float* q = allb + 5 * j;
+    const int staged = METRIC == TDS_METRIC_DISCS ? N + min(kRowsPerCta, A - row0) : N;
+    for (int j = threadIdx.x; j < staged; j += blockDim.x) {
+        const float* q = j < N ? allb + 5 * j : ego + ((size_t)b * A + row0 + (j - N)) * 5;
         float* s = smem + j * STRIDE;
         if (METRIC == TDS_METRIC_DISCS) {
             const Discs d = make_discs(q[0], q[1], q[2], q[3], q[4]);
 #pragma unroll
             for (int k = 0; k < kDiscs; k++) { s[2 * k] = d.cx[k]; s[2 * k + 1] = d.cy[k]; }
-            s[10] = d.r; s[11] = d.half; s[12] = mb[j] ? 1.0f : 0.0f;
+            s[10] = d.r; s[11] = d.half; s[12] = j >= N || mb[j] ? 1.0f : 0.0f;
         } else {
             const Box d = make_box(q[0], q[1], q[2], q[3], q[4]);
             s[0] = d.x; s[1] = d.y; s[2] = d.l; s[3] = d.w; s[4] = d.s; s[5] = d.c; s[6] = mb[j] ? 1.0f : 0.0f;
@@ -878,7 +881,13 @@ __global__ void __launch_bounds__(kWarps * 32) allpairs_fwd_kernel(const float* 
         float sum = 0.0f, best = -CUDART_INF_F;
         int besti = 0;
         if (METRIC == TDS_METRIC_DISCS) {
-            const Discs dp = make_discs(p[0], p[1], p[2], p[3], p[4]);
+            Discs dp;
+            {
+                const float* s = smem + (N + r) * STRIDE;
+#pragma unroll
+                for (int k = 0; k < kDiscs; k++) { dp.cx[k] = s[2 * k]; dp.cy[k] = s[2 * k + 1]; }
+                dp.r = s[10]; dp.half = s[11];
+            }
             for (int j = lane; j < N; j += 32) {
                 const float* s = smem + j * STRIDE;
                 Discs dq;
@@ -1169,8 +1178,10 @@ extern "C" int tds_collision_allpairs_fwd(const float* d_ego_box, const float* d
     TDS_REQUIRE(metric == TDS_METRIC_DISCS || metric == TDS_METRIC_IOU, "collision_allpairs: unknown metric %d", metric);
     TDS_REQUIRE(B <= 65535, "collision_allpairs: B=%d exceeds 65535 (shard the batch)", B);
     const dim3 grid((A + kRowsPerCta - 1) / kRowsPerCta, B);
-    const size_t smem = (size_t)N * (metric == TDS_METRIC_DISCS ? 13 : 7) * sizeof(float);
-    TDS_REQUIRE(smem <= 200 * 1024, "collision_allpairs: N=%d does not fit shared memory", N);
+    const size_t cols = (size_t)N * (metric == TDS_METRIC_DISCS ? 13 : 7) * sizeof(float);
+    TDS_REQUIRE(cols <= 200 * 1024, "collision_allpairs: N=%d does not fit shared memory", N);
+    // discs: the CTA's rows (at most 3.3 KB) come on top of the columns, within the 227 KB a CTA may have
+    const size_t smem = metric == TDS_METRIC_DISCS ? cols + (size_t)std::min(A, kRowsPerCta) * 13 * sizeof(float) : cols;
     const auto kernel = metric == TDS_METRIC_DISCS ? allpairs_fwd_kernel<TDS_METRIC_DISCS> : allpairs_fwd_kernel<TDS_METRIC_IOU>;
     if (int e = tds::allow_dynamic_smem(kernel, smem)) return e;
     kernel<<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(d_ego_box, d_all_box, d_mask, A, N, ego_is_prefix, d_out, d_argmax);

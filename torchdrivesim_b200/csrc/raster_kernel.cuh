@@ -554,6 +554,8 @@ __global__ void __launch_bounds__(G == 32 ? 128 : G, G <= 128 ? TDS_RASTER_MINB 
     const int tid = G == 32 ? (threadIdx.x & 31) : threadIdx.x;
     const int lane = threadIdx.x & 31;
     const int K = pal.n_classes;                // planes = draw ranks of the active classes
+    // behind a LEAN kernel: the redo list is nearly always empty, and then every CTA leaves before it builds its tables
+    if (!LEAN && a.cam_list && a.cam_list[0] == 0) return;
 
     // CTA-wide tables: colour per draw rank (0 = background), reciprocals of the row runs, class -> plane
     __shared__ float4 s_lut[TDS_MAX_CLASSES + 1];

@@ -1,7 +1,8 @@
 """CUDA-graph replay of the whole hot path.
 
 `GraphedHotPath` records ONE step of a `Simulator` (kinematic step -> egocentric birdviews -> collisions ->
-offroad) into a CUDA graph over static buffers and replays it with new actions.  The step consists of ~5 of
+offroad) into a CUDA graph over static buffers and replays it with new actions; collisions and offroad are a second
+branch of the graph that runs beside the birdviews.  The step consists of ~5 of
 our kernels plus a dozen tiny torch kernels; replaying a graph removes the eager-mode launch gaps between
 them (the reference has no equivalent: it is eager PyTorch + a Python loop per triangle).
 
@@ -57,6 +58,7 @@ class GraphedHotPath:
             self._goals.state = self._goals.state.to(torch.int64).contiguous().clone()
             self._goal_saved = (self._goals.mask.clone(), self._goals.state.clone())
         sim.kinematic_model.set_state(self.state)
+        self._side = torch.cuda.Stream(device=dev)
         # warm up on a side stream (allocator, lazily built map handles), then capture
         s = torch.cuda.Stream(device=dev)
         s.wait_stream(torch.cuda.current_stream(dev))
@@ -88,10 +90,19 @@ class GraphedHotPath:
         sim.kinematic_model.step(self.action, out=self.state)
         if self._goals is not None:
             self._goals.step(self.state, sim.internal_time, threshold=sim.cfg.waypoint_removal_threshold, in_place=True)
-        if self._render:
-            sim.render_egocentric(res=self._res, fov=self._fov, out=self.images)
-        sim.compute_collision(out=self.collision)
-        sim.compute_offroad(out=self.offroad)
+        if not self._render:
+            sim.compute_collision(out=self.collision)
+            sim.compute_offroad(out=self.offroad)
+            return
+        # collisions and offroad depend on the new state only: a second branch of the graph, beside the raster.  Neither
+        # touches the raster's scratch buffers, which the library keys by (device, stream) and finds on the main stream.
+        main = torch.cuda.current_stream()
+        self._side.wait_stream(main)
+        with torch.cuda.stream(self._side):
+            sim.compute_collision(out=self.collision)
+            sim.compute_offroad(out=self.offroad)
+        sim.render_egocentric(res=self._res, fov=self._fov, out=self.images)
+        main.wait_stream(self._side)
 
     def run(self, action: Tensor) -> Tuple[Optional[Tensor], Tensor, Tensor]:
         """One step with `action` [B,A,Ac] (device or pinned host tensor).  Returns the static output
